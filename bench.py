@@ -80,7 +80,15 @@ def parse_args():
                          "RainflowSeiDegradation.rainflow_length (carried across episodes, rainflow_sei_degradation.py:195) converges "
                          "to its running maximum within a few episodes, after which fewer cycles need a stress evaluation; "
                          "without settling a 20-step window runs 5 %% slower than a 960-step one, with it 1.7 %%")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed step returned (reward, done, obs, terminal_obs) "
+                         "as DIR/<name>.npy, for a fixed, seeded sample of env rows (env_index.npy) of at most 64 MiB in all; "
+                         "rank 0's envs when run on several GPUs")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of --impl ours; the reference arm materialises none")
     cf = CONFIGS[args.config]
     world = int(os.environ.get("WORLD_SIZE", "1"))
     if args.envs is None:
@@ -256,6 +264,29 @@ def run_reference(args):
     print(json.dumps(line), flush=True)
 
 
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(path, obs, rew, done, term):
+    """Write what fleet_step returned to its caller in the last step as float32 / float64 .npy files under `path`.
+
+    All envs' rows would exceed DUMP_BYTES at the benchmark's sizes (obs alone is 100 MB at cfg2), so the same fixed,
+    seeded sample of env rows is taken from every per-env output; env_index.npy lists it.  terminal_obs holds the rows
+    of the sampled envs that finished in that step, in sample order: the step writes no other row of it."""
+    import torch
+    E, D = obs.shape
+    row_bytes = 8 + 4 * (2 + 2 * D)                  # env_index (f64), reward and done (f32), obs and terminal_obs rows
+    rows = min(E, (DUMP_BYTES - (1 << 16)) // row_bytes)     # 64 KiB left for the .npy headers
+    idx = np.arange(E) if rows == E else np.sort(np.random.default_rng(0).choice(E, rows, replace=False))
+    sel = torch.from_numpy(idx).to(obs.device)
+    d = done.index_select(0, sel)
+    arrays = {"env_index": idx.astype(np.float64), "reward": rew.index_select(0, sel), "done": d.float(),
+              "obs": obs.index_select(0, sel), "terminal_obs": term.index_select(0, sel)[d.bool()]}
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), a.cpu().numpy() if torch.is_tensor(a) else a)
+
+
 def workload_config(args, built, D):
     return {"workload": f"{args.cfg['label']}; {args.envs} envs/GPU", "name": args.config,
             "envs_per_gpu": args.envs, "evs": args.evs, "obs_dim": D, "table_len": int(built.consts.table_len),
@@ -354,6 +385,8 @@ def main():
     ms_per_step = total_ms / K
     value = world * E * N * K / (total_ms * 1e-3)
     err = h.check_errors()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, obs, rew, done, term)   # before the kernel-timing pass below overwrites them
 
     # roofline of the dominant kernel (the step kernel): algorithmic bytes per launch / its average launch duration,
     # measured live with CUDA events around each launch (fleet_set_timing) in a second pass over the same workload;

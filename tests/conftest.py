@@ -10,12 +10,14 @@ if ROOT not in sys.path:
 
 def pytest_configure(config):
     config.addinivalue_line("markers", "gpu: needs a CUDA device (run on the B200 box with -m gpu)")
-    config.addinivalue_line("markers", "reference: needs /root/reference (build container only; skipped elsewhere)")
+    config.addinivalue_line("markers", "reference: compares with an unmodified FleetRL checkout named by "
+                                       "FLEETRL_REFERENCE_ROOT; skipped without one")
 
 
 def pytest_collection_modifyitems(config, items):
-    ref_ok = os.path.isdir("/root/reference/fleetrl")
-    skip_ref = pytest.mark.skip(reason="/root/reference not present")
+    from oracle.refshim import compat
+    ref_ok = compat.available()
+    skip_ref = pytest.mark.skip(reason="no unmodified FleetRL checkout at FLEETRL_REFERENCE_ROOT")
     for item in items:
         if "reference" in item.keywords and not ref_ok:
             item.add_marker(skip_ref)
