@@ -23,6 +23,7 @@ EXPORTS = [
     "fleet_field_info", "fleet_get_stats", "fleet_reset_stats", "fleet_check_errors", "fleet_launch_count",
     "fleet_device_bytes", "fleet_last_error", "fleet_set_timing", "fleet_get_timing", "fleet_step_kernel_name", "fleet_policy_actions", "fleet_policy_reset", "fleet_enable_charge_log",
     "fleet_debug_stress", "fleet_enable_log", "fleet_log_layout", "fleet_read_log", "fleet_state_bytes", "fleet_export_state", "fleet_import_state",
+    "fleet_launch_geometry",
 ]
 
 
@@ -73,6 +74,7 @@ def load_library(path: str = LIB_PATH):
     L.fleet_import_state.argtypes = [vp, vp, vp]
     L.fleet_step_kernel_name.argtypes = [vp]
     L.fleet_step_kernel_name.restype = C.c_char_p
+    L.fleet_launch_geometry.argtypes = [vp] + [C.POINTER(i32)] * 4
     L.fleet_set_timing.argtypes = [vp, i32]
     L.fleet_get_timing.argtypes = [vp, C.POINTER(C.c_double), C.POINTER(C.c_double), C.POINTER(i64)]
     L.fleet_last_error.argtypes = [vp]
@@ -283,6 +285,14 @@ class FleetStepHandle:
     def step_kernel_name(self):
         """Name of the step kernel fleet_create selected for this handle."""
         return self.lib.fleet_step_kernel_name(self._h).decode()
+
+    @property
+    def launch_geometry(self):
+        """dict(step_grid, step_tiles, envs_per_tile, post_grid): the launch geometry fleet_create chose (after the
+        FLEETSTEP_PF_GRID / FLEETSTEP_POST_GRID caps)."""
+        v = [C.c_int32(0) for _ in range(4)]
+        self._check(self.lib.fleet_launch_geometry(self._h, *[C.byref(x) for x in v]), "fleet_launch_geometry")
+        return dict(zip(("step_grid", "step_tiles", "envs_per_tile", "post_grid"), (x.value for x in v)))
 
     @property
     def launch_count(self):

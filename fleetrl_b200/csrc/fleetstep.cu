@@ -2419,6 +2419,17 @@ const char* fleet_step_kernel_name(const FleetHandle* h) {
     return h->use_pf ? (h->pf_v == 2 ? "fleet_step_pf_kernel<kV=2>" : "fleet_step_pf_kernel<kV=1>") : "fleet_step_kernel";
 }
 
+int fleet_launch_geometry(const FleetHandle* h, int32_t* step_grid, int32_t* step_tiles, int32_t* envs_per_tile,
+                          int32_t* post_grid) {
+    if (!h) return FLEET_E_INVALID;
+    const int B = h->use_pf ? h->p.pf_B : h->p.B;
+    if (step_grid) *step_grid = h->use_pf ? h->grid_pf : h->grid;
+    if (step_tiles) *step_tiles = h->use_pf ? h->p.pf_ntiles : h->grid;
+    if (envs_per_tile) *envs_per_tile = B;
+    if (post_grid) *post_grid = h->need_post ? h->grid_post : 0;
+    return FLEET_OK;
+}
+
 int fleet_set_timing(FleetHandle* h, int32_t enable) {
     if (!h) return FLEET_E_INVALID;
     CUDA_TRY(h, cudaSetDevice(h->device));
@@ -2756,6 +2767,9 @@ int fleet_create(const FleetConsts* consts, const FleetTables* tb, int32_t num_e
         if (per_sm < 1) per_sm = 1;
         const int64_t g = (int64_t)h->num_sms * per_sm;
         h->grid_post = (int)(g < E ? g : E);
+        // FLEETSTEP_POST_GRID=G (diagnostic, G >= 1) caps the grid so that every CTA fetches many work items per launch
+        const int cap = env_int("FLEETSTEP_POST_GRID", 0);
+        if (cap > 0 && cap < h->grid_post) h->grid_post = cap;
     }
     h->smem_step = sm;
     {
@@ -2796,6 +2810,10 @@ int fleet_create(const FleetConsts* consts, const FleetTables* tb, int32_t num_e
                 p.pf_off_stage = (int)align16((size_t)p.pf_off_obs + (size_t)kPfOut * p.pf_obs_b);
                 const int g = prop.multiProcessorCount * per_sm;
                 h->grid_pf = g < ntiles ? g : ntiles;
+                // FLEETSTEP_PF_GRID=G (diagnostic, G >= 1) caps the persistent grid so that every CTA runs many tiles: the
+                // steady state of the buffer rotation at test sizes
+                const int cap = env_int("FLEETSTEP_PF_GRID", 0);
+                if (cap > 0 && cap < h->grid_pf) h->grid_pf = cap;
                 h->use_pf = 1;
             }
             cudaGetLastError();

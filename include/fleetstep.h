@@ -282,6 +282,14 @@ int fleet_import_state(FleetHandle* h, const void* src_host, void* stream);
 int fleet_debug_stress(const double* eff_dev, const double* mean_dev, double* out_dev, int32_t n, void* stream);
 
 const char* fleet_step_kernel_name(const FleetHandle* h);   /* which step kernel fleet_create selected */
+
+/* Launch geometry fleet_create chose: CTAs of the step kernel, tiles it covers (envs_per_tile envs each; the persistent
+ * pf kernel loops over them with a stride of step_grid, the generic kernel runs one CTA per tile) and CTAs of the post
+ * kernel (0 when no post kernel runs).  Two diagnostic environment variables, read by fleet_create, cap the grids
+ * below what the occupancy query gives, so that each CTA iterates over many tiles / work items at test sizes:
+ * FLEETSTEP_PF_GRID (pf step kernel) and FLEETSTEP_POST_GRID (post kernel); unset or <= 0 means no cap. */
+int fleet_launch_geometry(const FleetHandle* h, int32_t* step_grid, int32_t* step_tiles, int32_t* envs_per_tile,
+                          int32_t* post_grid);
 int fleet_set_timing(FleetHandle* h, int32_t enable);
 int fleet_get_timing(FleetHandle* h, double* step_kernel_ms, double* post_kernel_ms, int64_t* steps);
 

@@ -1,16 +1,13 @@
 """GPU vs CPU-oracle parity on many envs with auto-reset, random starts and random actions (through the C ABI).
 
-Bit-exact (asserted with array_equal): done, time index, hours_left, target flags, SOC / soc_deg (see below), rainflow cycle
-counts / rainflow_length, observations (float32), terminal observations, start indices drawn by the device RNG.
-Tolerance: reward rel 1e-11 / abs 1e-10 (deterministic re-association of the per-env sum, exp), cashflow rel 1e-12 (regrouped revenue factor), SOH abs 1e-13, fd_cyc rel 1e-11.
+The per-step comparison and its tolerances are those of parity_util.run_vs_oracle.
 """
-import zlib
-
 import numpy as np
 import pytest
 import torch
 
 from oracle.oracle import OracleFleet
+from parity_util import make_case, run_vs_oracle
 from synth_tables import make_consts, make_tables
 
 pytestmark = pytest.mark.gpu
@@ -48,7 +45,10 @@ KERNELS = ([(n, "pf") for n in sorted(CASES) if CASES[n]["n_evs"] >= 8 and CASES
            # the two-vehicles-per-thread variant of the pf kernel (off by default, FLEETSTEP_PF_V=2) and the two-warp /
            # one-warp work items of the post kernel
            + [("lmd_50ev", "pf+v2"), ("ct_20ev_two_trips", "pf+v2+post64"), ("ut_10ev_e50", "pf+v2"), ("lmd_50ev_e36", "pf+post32"),
-              ("lmd_300ev", "generic+post32")])
+              ("lmd_300ev", "generic+post32")]
+           # pf rows run the instance without the charge log (the one bench.py and FleetVecEnv use); "+log" rows run the
+           # kLog instances of both vehicle widths; generic rows keep the charge log on throughout
+           + [("lmd_50ev", "pf+log"), ("lmd_50ev", "pf+v2+log"), ("lmd_9ev_norm_nocarry", "pf+log")])
 
 
 @pytest.mark.parametrize("name,kernel", KERNELS)
@@ -69,87 +69,11 @@ def test_gpu_vs_oracle(name, kernel, monkeypatch):
 
     cs = dict(CASES[name])
     E, steps = cs.pop("E"), cs.pop("steps")
-    over = cs.pop("over", {})
-    use_case = cs.pop("use_case")
-    episode_hours = cs.pop("episode_hours", 24)
-    sph = cs.get("sph", 4)
-    cap0 = dict(lmd=60.0, ut=50.0, ct=16.7)[use_case]
-    tables, T = make_tables(seed=zlib.crc32(name.encode()) % 1000, cap=cap0, **cs)   # stable across runs
-    if not over.get("include_building", 1):
-        tables = dict(tables, load=None)
-    if not over.get("include_pv", 1):
-        tables = dict(tables, pv=None)
-    consts = make_consts(tables, T, cs["n_evs"], sph=sph, episode_hours=episode_hours, use_case=use_case, **over)
-    N = cs["n_evs"]
-
+    consts, tables = make_case(name, **cs)
     orc = OracleFleet(consts, tables, E, env_id_offset=1000)
     gpu = FleetStepHandle(consts, tables, E, device=0, env_id_offset=1000)
-    dev = gpu.device
-    D = gpu.D
-    assert D == orc.D
-    rng = np.random.default_rng(7)
-
-    obs = torch.zeros((E, D), dtype=torch.float32, device=dev)
-    term = torch.full((E, D), -7.0, dtype=torch.float32, device=dev)
-    rew = torch.zeros(E, dtype=torch.float32, device=dev)
-    done = torch.zeros(E, dtype=torch.uint8, device=dev)
-
-    gpu.enable_charge_log(True)              # EvCharger's charge_log of every step (FLEET_F_CHARGE_LOG)
-    o_obs = orc.reset()                      # start indices from the counter RNG on both sides
-    gpu.reset(obs=obs)
-    np.testing.assert_array_equal(gpu.get("time_idx").cpu().numpy(), orc.get("time_idx"))
-    np.testing.assert_array_equal(obs.cpu().numpy(), o_obs)
-
-    exact = ["time_idx", "finish_idx", "hours_left", "target_soc", "rf_len", "n_cycles", "ep_count"]
-    # SOC / soc_deg are bit-exact for a given SOH.  Once a vehicle has been through a daily SEI evaluation its SOH agrees
-    # with the oracle to 1e-13 only (device pow/exp vs libm, and the incremental rainflow adds a vehicle's cycle
-    # stress terms in commit order, not list order), so its capacity and hence its SOC may differ in the last
-    # bit: exact equality is asserted where degradation cannot interfere, the stated 1e-12 otherwise.
-    soc_exact = (not consts.calc_degradation) or consts.deg_mode == 1
-    n_done = 0
-    for s in range(steps):
-        a = rng.uniform(-1, 1, (E, N)).astype(np.float32)
-        if s % 5 == 0:
-            a[rng.random((E, N)) < 0.3] = 0.0          # exact zeros: plateaus in the SOC history
-        if s % 7 == 0:
-            a[:] = 1.0                                  # everybody charges: overload penalties
-        o_obs, o_rew, o_cash, o_done, o_term = orc.step(a, want_terminal=True)
-        gpu.step(torch.from_numpy(a).to(dev), obs, rew, done, term)
-        g_done = done.cpu().numpy()
-        np.testing.assert_array_equal(g_done, o_done, err_msg=f"done step {s}")
-        for k in exact:
-            np.testing.assert_array_equal(gpu.get(k).cpu().numpy(), orc.get(k), err_msg=f"{k} step {s}")
-        for k in ("soc", "soc_deg"):
-            g_v, o_v = gpu.get(k).cpu().numpy(), orc.get(k)
-            if soc_exact:
-                np.testing.assert_array_equal(g_v, o_v, err_msg=f"{k} step {s}")
-            else:
-                np.testing.assert_allclose(g_v, o_v, rtol=0, atol=1e-12, err_msg=f"{k} step {s}")
-                assert (g_v != o_v).mean() < 1e-2, f"{k} step {s}: too many non-identical elements"
-        g_cl, o_cl = gpu.get("charge_log").cpu().numpy(), orc.get("charge_log")
-        if soc_exact:
-            np.testing.assert_array_equal(g_cl, o_cl, err_msg=f"charge_log step {s}")
-        else:
-            np.testing.assert_allclose(g_cl, o_cl, rtol=0, atol=1e-10, err_msg=f"charge_log step {s}")
-        np.testing.assert_allclose(gpu.get("reward64").cpu().numpy(), o_rew, rtol=1e-11, atol=1e-10, err_msg=f"reward step {s}")
-        np.testing.assert_allclose(gpu.get("cashflow").cpu().numpy(), o_cash, rtol=1e-12, atol=1e-13)
-        np.testing.assert_allclose(rew.cpu().numpy(), o_rew.astype(np.float32), rtol=1e-6, atol=1e-6)
-        np.testing.assert_allclose(gpu.get("soh").cpu().numpy(), orc.get("soh"), rtol=0, atol=1e-13, err_msg=f"soh step {s}")
-        np.testing.assert_allclose(gpu.get("fd_cyc").cpu().numpy(), orc.get("fd_cyc"), rtol=1e-11, atol=1e-18)
-        np.testing.assert_allclose(gpu.get("life").cpu().numpy(), orc.get("life"), rtol=0, atol=1e-13)
-        np.testing.assert_allclose(gpu.get("overload").cpu().numpy(), orc.get("overload"), rtol=1e-12, atol=1e-12)
-        np.testing.assert_allclose(gpu.get("soc_viol").cpu().numpy(), orc.get("soc_viol"), rtol=1e-12, atol=1e-15)
-        np.testing.assert_array_equal(obs.cpu().numpy(), o_obs, err_msg=f"obs step {s}")
-        if consts.auto_reset and o_done.any():
-            idx = np.nonzero(o_done)[0]
-            np.testing.assert_array_equal(term.cpu().numpy()[idx], o_term[idx], err_msg=f"terminal obs step {s}")
-            n_done += len(idx)
-    if consts.auto_reset:
-        assert n_done > 0
-    g_stats, o_stats = gpu.stats(), orc.stats()
-    for k in o_stats:
-        np.testing.assert_allclose(g_stats[k], o_stats[k], rtol=1e-9, atol=1e-9, err_msg=f"stat {k}")
-    assert gpu.check_errors() == 0 and orc.err_flags() == 0
+    charge_log = kernel.startswith("generic") or "+log" in kernel
+    run_vs_oracle(gpu, orc, steps, charge_log=charge_log)
     gpu.close()
 
 
