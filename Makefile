@@ -5,10 +5,11 @@ NVCCFLAGS = $(ARCH) -O3 -lineinfo -std=c++17 -fmad=false -Xcompiler -fPIC,-ffp-c
 LIB = fleetrl_b200/libfleetstep.so
 
 all: $(LIB) oracle
-$(LIB): fleetrl_b200/csrc/fleetstep.cu include/fleetstep.h
-	$(NVCC) $(NVCCFLAGS) -Xptxas -v -shared -o $@ fleetrl_b200/csrc/fleetstep.cu
+SRCS = fleetrl_b200/csrc/fleetstep.cu fleetrl_b200/csrc/vecnorm.cu
+$(LIB): $(SRCS) include/fleetstep.h
+	$(NVCC) $(NVCCFLAGS) -Xptxas -v -shared -o $@ $(SRCS)
 timing:   # diagnostic build with per-phase cycle counters in the post kernel (scripts/post_timing.py)
-	$(NVCC) $(NVCCFLAGS) -DPOST_TIMING -shared -o fleetrl_b200/libfleetstep_timing.so fleetrl_b200/csrc/fleetstep.cu
+	$(NVCC) $(NVCCFLAGS) -DPOST_TIMING -shared -o fleetrl_b200/libfleetstep_timing.so $(SRCS)
 oracle:
 	$(MAKE) -C oracle
 clean:

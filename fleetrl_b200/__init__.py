@@ -10,6 +10,9 @@ def __getattr__(name):  # lazy: importing the package must not require torch / C
     if name in ("FleetVecEnv", "FleetEnv", "LazyInfos"):
         from . import vec_env
         return getattr(vec_env, name)
+    if name == "FleetVecNormalize":
+        from . import normalize
+        return normalize.FleetVecNormalize
     if name in ("build_fleet", "FleetInputs"):
         from . import tables
         return getattr(tables, name)

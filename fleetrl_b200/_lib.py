@@ -24,6 +24,8 @@ EXPORTS = [
     "fleet_device_bytes", "fleet_last_error", "fleet_set_timing", "fleet_get_timing", "fleet_step_kernel_name", "fleet_policy_actions", "fleet_policy_reset", "fleet_enable_charge_log",
     "fleet_debug_stress", "fleet_enable_log", "fleet_log_layout", "fleet_read_log", "fleet_state_bytes", "fleet_export_state", "fleet_import_state",
     "fleet_launch_geometry",
+    "fleet_norm_create", "fleet_norm_destroy", "fleet_norm_set_flags", "fleet_norm_moments_len", "fleet_norm_moments",
+    "fleet_norm_apply", "fleet_norm_reset_returns", "fleet_norm_get_state", "fleet_norm_set_state", "fleet_norm_last_error",
 ]
 
 
@@ -79,6 +81,18 @@ def load_library(path: str = LIB_PATH):
     L.fleet_get_timing.argtypes = [vp, C.POINTER(C.c_double), C.POINTER(C.c_double), C.POINTER(i64)]
     L.fleet_last_error.argtypes = [vp]
     L.fleet_last_error.restype = C.c_char_p
+    f64 = C.c_double
+    L.fleet_norm_create.argtypes = [i32, i32, i32, f64, f64, f64, f64, C.POINTER(vp)]
+    L.fleet_norm_destroy.argtypes = [vp]
+    L.fleet_norm_set_flags.argtypes = [vp, i32, i32, i32]
+    L.fleet_norm_moments_len.argtypes = [vp]
+    L.fleet_norm_moments.argtypes = [vp, vp, vp, vp, vp]
+    L.fleet_norm_apply.argtypes = [vp, vp, i64] + [vp] * 8
+    L.fleet_norm_reset_returns.argtypes = [vp, vp]
+    L.fleet_norm_get_state.argtypes = [vp] * 9
+    L.fleet_norm_set_state.argtypes = [vp] * 9
+    L.fleet_norm_last_error.argtypes = [vp]
+    L.fleet_norm_last_error.restype = C.c_char_p
     if L.fleet_abi_version() != ABI_VERSION:
         raise FleetStepError("libfleetstep.so ABI version does not match fleetrl_b200/_abi.py")
     _LIB = L
@@ -305,3 +319,102 @@ class FleetStepHandle:
     @property
     def raw(self):
         return self._h
+
+
+class FleetNormHandle:
+    """Device VecNormalize statistics for [E][D] float32 batches (fleet_norm_*): thin, checked wrapper over the C ABI."""
+
+    def __init__(self, num_envs: int, obs_dim: int, device=0, clip_obs=10.0, clip_reward=10.0, gamma=0.99, epsilon=1e-8):
+        if not torch.cuda.is_available():
+            raise FleetStepError("no CUDA device available; fleetrl_b200 has no CPU fallback")
+        self.lib = load_library()
+        self.device = torch.device("cuda", device if isinstance(device, int) else torch.device(device).index or 0)
+        h = C.c_void_p()
+        rc = self.lib.fleet_norm_create(int(num_envs), int(obs_dim), self.device.index, float(clip_obs), float(clip_reward),
+                                        float(gamma), float(epsilon), C.byref(h))
+        self._h = h
+        if rc != 0:
+            msg = self.lib.fleet_norm_last_error(h).decode() if h else "fleet_norm_create failed"
+            if h:
+                self.lib.fleet_norm_destroy(h)
+            self._h = None
+            raise FleetStepError(f"fleet_norm_create: {msg} (code {rc})")
+        self.E, self.D = int(num_envs), int(obs_dim)
+        self.moments_len = int(self.lib.fleet_norm_moments_len(h))
+
+    def close(self):
+        if getattr(self, "_h", None):
+            self.lib.fleet_norm_destroy(self._h)
+            self._h = None
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+    def _check(self, rc, what):
+        if rc != 0:
+            raise FleetStepError(f"{what}: {self.lib.fleet_norm_last_error(self._h).decode()} (code {rc})")
+
+    _chk_tensor = FleetStepHandle._chk_tensor
+
+    def set_flags(self, training, norm_obs, norm_reward):
+        self._check(self.lib.fleet_norm_set_flags(self._h, int(bool(training)), int(bool(norm_obs)), int(bool(norm_reward))),
+                    "fleet_norm_set_flags")
+
+    def moments(self, obs, reward, out):
+        """Batch moments of obs [E, D] (and of the new returns when reward [E] is given) into out (float64 [2D+4])."""
+        self._chk_tensor(obs, (self.E, self.D), torch.float32, "obs")
+        self._chk_tensor(reward, (self.E,), torch.float32, "reward")
+        self._chk_tensor(out, (self.moments_len,), torch.float64, "moments")
+        if out is None:
+            raise FleetStepError("moments: an output tensor is required")
+        self._check(self.lib.fleet_norm_moments(self._h, _dptr(obs), _dptr(reward), _dptr(out), _stream_ptr(self.device)),
+                    "fleet_norm_moments")
+
+    def apply(self, moments=None, obs=None, obs_out=None, reward=None, reward_out=None, done=None, terminal_obs=None,
+              terminal_obs_out=None):
+        """Merge `moments` (None: no update) and normalise; see fleet_norm_apply."""
+        rows = next((t.shape[0] for t in (obs, reward, done) if t is not None), self.E)
+        self._chk_tensor(moments, (self.moments_len,), torch.float64, "moments")
+        for t, nm in ((obs, "obs"), (obs_out, "obs_out"), (terminal_obs, "terminal_obs"), (terminal_obs_out, "terminal_obs_out")):
+            self._chk_tensor(t, (rows, self.D), torch.float32, nm)
+        self._chk_tensor(reward, (rows,), torch.float32, "reward")
+        self._chk_tensor(reward_out, (rows,), torch.float32, "reward_out")
+        self._chk_tensor(done, (rows,), torch.uint8, "done")
+        self._check(self.lib.fleet_norm_apply(self._h, _dptr(moments), int(rows), _dptr(obs), _dptr(obs_out), _dptr(reward),
+                                              _dptr(reward_out), _dptr(done), _dptr(terminal_obs), _dptr(terminal_obs_out),
+                                              _stream_ptr(self.device)), "fleet_norm_apply")
+
+    def reset_returns(self):
+        self._check(self.lib.fleet_norm_reset_returns(self._h, _stream_ptr(self.device)), "fleet_norm_reset_returns")
+
+    STATE = ("obs_mean", "obs_var", "obs_count", "ret_mean", "ret_var", "ret_count", "returns")
+
+    def _shapes(self):
+        return ((self.D,), (self.D,), (), (), (), (), (self.E,))
+
+    def get_state(self):
+        """dict of float64 NumPy arrays: obs_mean [D], obs_var [D], obs_count, ret_mean, ret_var, ret_count, returns [E]."""
+        out = {k: np.zeros(s, np.float64) for k, s in zip(self.STATE, self._shapes())}
+        self._check(self.lib.fleet_norm_get_state(self._h, *[out[k].ctypes.data for k in self.STATE], _stream_ptr(self.device)),
+                    "fleet_norm_get_state")
+        return out
+
+    def set_state(self, **parts):
+        """Set any of the get_state() entries; the others stay."""
+        bad = set(parts) - set(self.STATE)
+        if bad:
+            raise KeyError(f"unknown state entries {sorted(bad)}")
+        keep = {}
+        for k, s in zip(self.STATE, self._shapes()):
+            if parts.get(k) is not None:
+                a = np.array(parts[k], dtype=np.float64, order="C")
+                if a.shape != s and a.size == 1 and s == ():
+                    a = a.reshape(())
+                if a.shape != s:
+                    raise FleetStepError(f"{k}: expected shape {s}, got {a.shape}")
+                keep[k] = a
+        self._check(self.lib.fleet_norm_set_state(self._h, *[keep[k].ctypes.data if k in keep else None for k in self.STATE],
+                                                  _stream_ptr(self.device)), "fleet_norm_set_state")

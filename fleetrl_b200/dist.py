@@ -1,6 +1,7 @@
-"""Multi-GPU plumbing: environments shard across ranks with no data-path collective; the only exchange is one
+"""Multi-GPU plumbing: environments shard across ranks with no data-path collective; the exchanges are one
 all-reduce of the episode-statistics vector (the columns of the reference's DataLogger row, data_logger.py:55-68,
-summed over envs) per rollout / report.  torch.distributed over NCCL on GPUs (gloo in the CPU tests)."""
+summed over envs) per rollout / report and, under FleetVecNormalize, one all-reduce of its batch-moments vector per
+step.  torch.distributed over NCCL on GPUs (gloo in the CPU tests)."""
 import os
 
 import torch
@@ -30,3 +31,9 @@ def all_reduce_stats(stats: torch.Tensor) -> torch.Tensor:
     if dist is not None and dist.is_available() and dist.is_initialized() and dist.get_world_size() > 1:
         dist.all_reduce(stats, op=dist.ReduceOp.SUM)
     return stats
+
+
+def all_reduce_moments(moments: torch.Tensor) -> torch.Tensor:
+    """Sum FleetVecNormalize's batch moments (float64 [2D+4], shifted sums about the running means every rank holds
+    identically) over all ranks, in place, so that every rank merges the same global batch into its statistics."""
+    return all_reduce_stats(moments)

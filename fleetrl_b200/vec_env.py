@@ -152,7 +152,9 @@ class FleetVecEnv(_VecEnvBase):
         self.step_async(actions)
         return self.step_wait()
 
-    def _infos(self, done_idx):
+    def _infos(self, done_idx, terminal_obs=None):
+        """infos of the step just taken; terminal_obs: the [E, D] buffer holding the terminal rows (default: this env's
+        own, a wrapper passes its normalised copy)."""
         if done_idx is None:   # torch mode: one small D2H of the done flags (use step_raw() to avoid it)
             done_idx = torch.nonzero(self._done).flatten().cpu().numpy()
             self._last_done = np.zeros(self.num_envs, dtype=bool)
@@ -160,7 +162,7 @@ class FleetVecEnv(_VecEnvBase):
         if len(done_idx) == 0:
             return LazyInfos(self.num_envs, [], None, None, 0)
         idx_t = torch.as_tensor(done_idx, device=self.device, dtype=torch.long)
-        term = self._term.index_select(0, idx_t)          # terminal rows of the finished envs only
+        term = (self._term if terminal_obs is None else terminal_obs).index_select(0, idx_t)   # finished envs' rows only
         if self.output == "numpy":
             term = term.cpu().numpy()
         rets = self.handle.get("last_ep_return").index_select(0, idx_t).cpu().numpy()

@@ -298,6 +298,67 @@ int64_t fleet_device_bytes(const FleetHandle* h);
 
 const char* fleet_last_error(const FleetHandle* h);
 
+/*
+ * FleetNorm — SB3 2.3.2's VecNormalize (stable_baselines3/common/vec_env/vec_normalize.py) with its two RunningMeanStd
+ * (common/running_mean_std.py) on the device, for any [E][D] float32 observation batch.  Independent of FleetHandle:
+ * like SB3, the statistics live apart from the env and are saved separately.  Same arithmetic and defaults: float64
+ * statistics, count 1e-4 / mean 0 / var 1 at creation, obs -> float32(clip((x - mean) / sqrt(var + eps), +-clip_obs)),
+ * reward -> clip(reward / sqrt(ret_var + eps), +-clip_reward) as float32.  A training step is two calls:
+ *   fleet_norm_moments  batch moments into a caller-owned float64 vector of fleet_norm_moments_len entries;
+ *   (multi-GPU: all-reduce that vector with SUM: every rank holds the same statistics, so the sums add)
+ *   fleet_norm_apply    merges them into the statistics and writes the normalised outputs.
+ * One kernel launch each, no host synchronisation.  The batch moments are computed in float64 where SB3 reduces
+ * in the observation dtype (float32): the statistics differ from SB3's at float32 rounding level.
+ */
+typedef struct FleetNorm FleetNorm;
+
+/* Replaces VecNormalize.__init__ (vec_normalize.py) for num_envs envs with obs_dim observations on GPU `device`.
+ * FLEET_E_INVALID for sizes < 1, clip_obs or clip_reward <= 0, gamma outside [0, 1], epsilon < 0.  *out is set
+ * even on failure (fleet_norm_last_error); the caller destroys it. */
+int fleet_norm_create(int32_t num_envs, int32_t obs_dim, int32_t device, double clip_obs, double clip_reward, double gamma,
+                      double epsilon, FleetNorm** out);
+int fleet_norm_destroy(FleetNorm* n);
+
+/* The attributes VecNormalize.training / norm_obs / norm_reward (vec_normalize.py).  Initially all 1. */
+int fleet_norm_set_flags(FleetNorm* n, int32_t training, int32_t norm_obs, int32_t norm_reward);
+
+/* Length 2*obs_dim+4 of the moments vector: {obs n, sum(x-K)[D], sum((x-K)^2)[D], ret n, sum(r-Kr), sum((r-Kr)^2)}
+ * with K, Kr the current running means and r = returns*gamma + reward the new returns. */
+int fleet_norm_moments_len(const FleetNorm* n);
+
+/* The data half of RunningMeanStd.update (running_mean_std.py) for obs_rms (VecNormalize.step_wait's
+ * obs_rms.update(obs), vec_normalize.py; reset's _update_obs) and, when reward_dev is given, for ret_rms
+ * (_update_reward, :236-239).  obs_dev float32 [E][D], reward_dev float32 [E] or NULL.  The obs part is computed only when
+ * training and norm_obs, the returns part only when training; a part not computed has n = 0.  No side effects: writes
+ * moments_dev only.  Deterministic: independent of the grid and of the SM count. */
+int fleet_norm_moments(FleetNorm* n, const float* obs_dev, const float* reward_dev, double* moments_dev, void* stream);
+
+/* The rest of VecNormalize.step_wait (vec_normalize.py) / reset and normalize_obs /
+ * normalize_reward  on `rows` rows:
+ *   moments_dev (ignored unless training): merged into the statistics with update_from_moments (running_mean_std.py);
+ *               with rewards, also returns = returns*gamma + reward.  NULL: normalise with the current statistics only.
+ *   obs_dev -> obs_out_dev        float32 [rows][D], normalised when norm_obs, else copied; obs_dev stays intact
+ *   reward_dev -> reward_out_dev  float32 [rows], normalised when norm_reward, else copied
+ *   done_dev uint8 [E]: returns[done] = 0, and terminal_obs_dev rows of finished envs are normalised into
+ *               terminal_obs_out_dev (other rows untouched), with the statistics after this call's update.
+ * Any pointer pair may be NULL.  A statistics update or done_dev requires rows == E.  Views need not be 16-byte aligned. */
+int fleet_norm_apply(FleetNorm* n, const double* moments_dev, int64_t rows, const float* obs_dev, float* obs_out_dev,
+                     const float* reward_dev, float* reward_out_dev, const uint8_t* done_dev, const float* terminal_obs_dev,
+                     float* terminal_obs_out_dev, void* stream);
+
+/* self.returns = np.zeros(self.num_envs) of VecNormalize.reset (vec_normalize.py). */
+int fleet_norm_reset_returns(FleetNorm* n, void* stream);
+
+/* obs_rms.mean/var/count [D]/[D]/1, ret_rms.mean/var/count 1/1/1 and returns [E] as float64 HOST arrays (the attributes
+ * VecNormalize.save pickles, vec_normalize.py).  A NULL pointer skips that part.  Both synchronise. */
+int fleet_norm_get_state(FleetNorm* n, double* obs_mean, double* obs_var, double* obs_count, double* ret_mean,
+                         double* ret_var, double* ret_count, double* returns, void* stream);
+int fleet_norm_set_state(FleetNorm* n, const double* obs_mean, const double* obs_var, const double* obs_count,
+                         const double* ret_mean, const double* ret_var, const double* ret_count, const double* returns,
+                         void* stream);
+
+const char* fleet_norm_last_error(const FleetNorm* n);
+
 #ifdef __cplusplus
 }
 #endif
