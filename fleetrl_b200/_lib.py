@@ -208,6 +208,13 @@ class FleetStepHandle:
         fid, dt, per_ev = FIELDS[name]
         v = torch.as_tensor(value, dtype=_TORCH_DTYPES[dt], device=self.device).contiguous()
         self._chk_tensor(v, (self.E, self.N) if per_ev else (self.E,), _TORCH_DTYPES[dt], name)
+        if name == "target_soc":
+            # the device keeps a vehicle's target as one flag: raised to 0.9 (fleet_environment.py:613-614) or not
+            target = float(self.consts.target_soc)
+            bad = (v != 0.9) & (v != target)
+            if bool(bad.any()):
+                raise FleetStepError(f"set(target_soc): {v[bad][0].item()!r} is neither the configured target {target!r} "
+                                     "nor 0.9, the only values a vehicle's target can take")
         self._check(self.lib.fleet_set_state(self._h, fid, _dptr(v), _stream_ptr(self.device)), f"fleet_set_state({name})")
         torch.cuda.current_stream(self.device).synchronize()
 

@@ -115,7 +115,12 @@ enum {
     FLEET_F_HOURS_LEFT = 1,  /* float  [E][N]  Episode.hours_left            episode.py:29                     */
     FLEET_F_SOC_DEG = 2,     /* double [E][N]  Episode.soc_deg               episode.py:23                     */
     FLEET_F_SOH = 3,         /* double [E][N]  Episode.soh                   episode.py:28                     */
-    FLEET_F_TARGET_SOC = 4,  /* double [E][N]  FleetEnv.target_soc           fleet_environment.py:263,613      */
+    FLEET_F_TARGET_SOC = 4,  /* double [E][N]  FleetEnv.target_soc           fleet_environment.py:263,613      *
+                              *                 Only two values exist: the configured target, or 0.9 once the vehicle's
+                              *                 SOH has fallen to <= 0.9.  fleet_set_state stores one flag per vehicle,
+                              *                 set where the value is 0.9 (and the target is not), and recounts the
+                              *                 flags; any other value reads back as the configured target.
+                              *                 FleetStepHandle.set rejects such values.                               */
     FLEET_F_TIME_IDX = 5,    /* int32  [E]     index of Episode.time in the table                              */
     FLEET_F_FINISH_IDX = 6,  /* int32  [E]     index of Episode.finish_time                                    */
     FLEET_F_REWARD64 = 7,    /* double [E]     reward of the last step before the f32 cast                     */
@@ -214,7 +219,9 @@ int fleet_step_host(FleetHandle* h, const float* actions_host, float* obs_host, 
 int fleet_set_next_start(FleetHandle* h, const int32_t* next_start_idx_dev);
 
 /* Copy one state field (FLEET_F_*) device-to-device into / out of caller memory; backs env_method() helpers
- * (fleet_environment.py:741-799), tests and state_dict()/load_state_dict(). */
+ * (fleet_environment.py:741-799), tests and state_dict()/load_state_dict().  FLEET_F_SOC_DEG, FLEET_F_TIME_IDX,
+ * FLEET_F_FINISH_IDX and FLEET_F_EP_COUNT are read-only; FLEET_F_TARGET_SOC stores, per vehicle, whether the value
+ * is 0.9 (see the field). */
 int fleet_get_state(FleetHandle* h, int32_t field, void* dst_dev, void* stream);
 int fleet_set_state(FleetHandle* h, int32_t field, const void* src_dev, void* stream);
 /* Element size in bytes and element count ([E][N] or [E]) of a field. */
@@ -271,7 +278,8 @@ int fleet_read_log(FleetHandle* h, double* rows_host, int64_t* counts_host, void
 /* Checkpoint / resume: the complete env state of the handle (time indices, SOC, SOH, history ring, rainflow stacks,
  * degradation members, statistics) as one opaque blob of fleet_state_bytes bytes in host memory.  fleet_import_state only
  * accepts a blob exported from a handle created with the same configuration and num_envs.  Both synchronise.
- * Backs FleetVecEnv.state_dict() / load_state_dict(). */
+ * Backs FleetVecEnv.state_dict() / load_state_dict().  The night policy's window state (fleet_policy_actions) belongs
+ * to the caller's evaluation loop, not to the envs: it is not in the blob (fleet_policy_reset clears it). */
 int64_t fleet_state_bytes(FleetHandle* h);
 int fleet_export_state(FleetHandle* h, void* dst_host, void* stream);
 int fleet_import_state(FleetHandle* h, const void* src_host, void* stream);

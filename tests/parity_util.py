@@ -78,12 +78,15 @@ def mixed_tiles(done, B):
     return int(((fin > 0) & (run > 0)).sum())
 
 
-def run_vs_oracle(gpu, orc, steps, *, charge_log, dephase=0, outputs=None, action_seed=7):
+def run_vs_oracle(gpu, orc, steps, *, charge_log, dephase=0, outputs=None, action_seed=7, hook=None):
     """Reset both sides through the counter RNG, then step them with the same random actions and compare every output
     and state field after every step.
 
     dephase=L: after each of the first L steps, env e with e % L == s is reset again (masked reset on both sides), so
     that episodes end on different steps (the de-phased steady state of a long rollout).
+    hook(s, actions, obs, reward, done, terminal_obs), if given, runs after the reset (s = -1, actions and step outputs
+    None) and at the end of every step s, once that step has been compared: it may write state on both sides or step
+    further handles with the same actions.
     Returns dict(n_done, mixed_tiles): finished episodes, and tiles (of the handle's launch geometry) that had finishing
     and running envs in the same step."""
     E, N, D = gpu.E, gpu.N, gpu.D
@@ -103,6 +106,8 @@ def run_vs_oracle(gpu, orc, steps, *, charge_log, dephase=0, outputs=None, actio
     gpu.reset(obs=obs0)
     np.testing.assert_array_equal(gpu.get("time_idx").cpu().numpy(), orc.get("time_idx"))
     np.testing.assert_array_equal(obs0.cpu().numpy(), o_obs)
+    if hook:
+        hook(-1, None, obs0, None, None, None)
 
     # SOC / soc_deg are bit-exact for a given SOH.  Once a vehicle has been through a daily SEI evaluation its SOH agrees
     # with the oracle to 1e-13 only (device pow/exp vs libm, and the incremental rainflow adds a vehicle's cycle
@@ -161,6 +166,8 @@ def run_vs_oracle(gpu, orc, steps, *, charge_log, dephase=0, outputs=None, actio
             if obs is not None:
                 np.testing.assert_array_equal(obs.cpu().numpy()[idx], o_r[idx], err_msg=f"reset obs step {s}")
         io.check_untouched(s)
+        if hook:
+            hook(s, a, obs, rew, done, term)
     if consts.auto_reset:
         assert n_done > 0
     g_stats, o_stats = gpu.stats(), orc.stats()
