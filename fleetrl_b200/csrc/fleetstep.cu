@@ -134,7 +134,9 @@ struct StepParams {
     unsigned int* err_flags;  // [1]
     const int* next_start;    // [E] or nullptr
     int2* wl;                 // [E] work list of the post kernel: {env, WL_* flags}
-    int* wl_count;            // [4] {entries pushed from the front, next entry to fetch, entries pushed from the back, -}
+    int4* wl_flush;           // [E] flush-only entries of the post kernel: {env, k_done, k_now, -}
+    int* wl_count;            // [8] {entries pushed from the front, next entry to fetch, entries pushed from the back,
+                              //      flush-only entries, next flush unit to fetch, -, -, -}
     unsigned int* wl_done;    // [1]
     int* wl_chunks;           // [E] per work-list entry: chunks of it that have finished (self-clearing), or nullptr
     int post_chunks, post_cv; // post kernel: work items per entry, vehicles per item
@@ -338,17 +340,20 @@ __device__ __forceinline__ void reset_slot(const StepParams& p, int e, int n, in
 // of the stack is always the most recently yielded reversal), reversals are pushed, closed cycles are committed.
 // An evaluation then pushes the provisional end point onto a READ-ONLY view of the stack and counts the residue.
 #ifdef POST_TIMING   // diagnostic build: cycles per phase of the post kernel, taken by thread 0 of every CTA (scripts/post_timing.py)
+// (slots 1-14: work-list entries; slot 15: flush units, slot 0: their cycles, taken by lane 0 of every warp)
 __device__ unsigned long long g_post_clk[16];
 #ifdef POST_TIMING_EVAL_ONLY   /* only the entries with a daily evaluation are timed */
 #define PT_ON(c_) (c_)
 #else
 #define PT_ON(c_) true
 #endif
-#define PT_START(c_) long long _pt = clock64(); const bool _pt_on = PT_ON(c_)
+#define PT_START2(k_, c_) long long _pt = clock64(); const bool _pt_on = (k_) && PT_ON(c_)
+#define PT_START(c_) PT_START2(true, c_)
 #define PT_MARK(k) do { if (threadIdx.x == 0 && _pt_on) { const long long _c = clock64(); atomicAdd(&g_post_clk[k], (unsigned long long)(_c - _pt)); _pt = _c; } } while (0)
 #define PT_COUNT(k, n) do { if (threadIdx.x == 0 && _pt_on) atomicAdd(&g_post_clk[k], (unsigned long long)(n)); } while (0)
 #else
 #define PT_START(c_) do {} while (0)
+#define PT_START2(k_, c_) do {} while (0)
 #define PT_MARK(k) do {} while (0)
 #define PT_COUNT(k, n) do {} while (0)
 #endif
@@ -592,8 +597,9 @@ __device__ __noinline__ double rf_vehicle_slow(const StepParams& p, int e, int n
     return deg;
 }
 
-// FAST path, one vehicle per thread of a post-kernel entry, WARP-SYNCHRONOUS (all 32 lanes call it; `active` = the lane
-// has a vehicle): consume history samples k_done+1 .. k_now, then (evaluate) run calculate_degradation.
+// FAST path, one vehicle per lane, WARP-SYNCHRONOUS (all 32 lanes call it; `active` = the lane has a vehicle): consume
+// history samples k_done+1 .. k_now, then (kEval && evaluate) run calculate_degradation.  e, k_done and k_now may differ
+// from lane to lane (flush units span envs); `evaluate` must be uniform over the warp.
 //   smcol   this thread's column of the stack copy: entry s at smcol[s * kPostThreads], s < S (a vehicle whose stack is
 //           or gets deeper leaves for rf_vehicle_slow with its HBM state untouched); the top two entries are carried in
 //           registers (t1 = top, t2 = below) together with Y = |t1 - t2| (+inf while there is only one point)
@@ -607,7 +613,7 @@ __device__ __noinline__ double rf_vehicle_slow(const StepParams& p, int e, int n
 // run inside that loop: cycles that need them are appended to the warp's list, which all 32 lanes evaluate together
 // (one cycle per lane, whoever owns it); each owner then adds up its own results in list order (deterministic).
 // Returns the SOH loss (0 unless evaluated).
-template <int kT>
+template <int kT, bool kEval>
 __device__ __forceinline__ double rf_vehicle(const StepParams& p, int e, int n, bool active, int k_done, int k_now,
                                              bool evaluate, double s_temp, double* __restrict__ smcol,
                                              double* __restrict__ qcol, double2* __restrict__ pcol) {
@@ -633,7 +639,7 @@ __device__ __forceinline__ double rf_vehicle(const StepParams& p, int e, int n, 
     }
     bool slow = active && depth > S;                         // this lane's vehicle takes the general path
     bool live = active && !slow;
-    PT_START(evaluate);
+    PT_START2(kEval, evaluate);
     double t1 = 0, t2 = 0, Y = inf;
     if (live) {
         t1 = smcol[(depth - 1) * kT];
@@ -669,7 +675,7 @@ __device__ __forceinline__ double rf_vehicle(const StepParams& p, int e, int n, 
     // ---- committed part: rainflow.reversals + extract_cycles over the pending samples
     int nq = 0;                                              // queued reversals
     for (int r0 = k_done + 1; ; r0 += kRfBatch) {
-        const bool more = r0 <= k_now;                       // (uniform over the CTA)
+        const bool more = r0 <= k_now;                       // (lanes with fewer pending rows run on with d == 0)
         // extract_cycles(): empty the queues when the next batch might not fit, and after the last row
         if (__any_sync(full, more ? nq > kRfQueue - kRfBatch : nq > 0)) {
             PT_MARK(2);
@@ -710,7 +716,7 @@ __device__ __forceinline__ double rf_vehicle(const StepParams& p, int e, int n, 
             nq = 0;
             PT_MARK(3);
         }
-        if (!more) break;
+        if (!__any_sync(full, more)) break;
         // reversals(): eight rows in flight, lock-step over the lanes, no branches.  Rows past k_now repeat the last
         // sample (d == 0: nothing happens); d_last * d_next < 0 is the reference's own test.
         double xb[kRfBatch];
@@ -732,7 +738,7 @@ __device__ __forceinline__ double rf_vehicle(const StepParams& p, int e, int n, 
 
     // ---- evaluation: the provisional end point x_cur on a READ-ONLY view stack[lo .. h) of the committed points
     double deg = 0;
-    if (evaluate) {                                          // (uniform over the CTA)
+    if (kEval && evaluate) {                                 // (uniform over the warp)
         const int len = k_now + 1;                           // samples in the reference's soc_log
         int m = c, h = depth, lo = 0, k = 0;
         double msum = acc.x, fs = 0;
@@ -943,9 +949,12 @@ __device__ __forceinline__ void ev_slot_step(const StepParams& p, const EnvT& es
 constexpr int WL_TRIGGER = 1, WL_RESET = 2, WL_FLUSH = 4;
 // Entries with a daily evaluation are by far the longest (consumption + residue stress + fade): they are pushed from the
 // front of the list and fetched first by the post kernel, everything else from the back, so that the kernel does not end
-// with one late-started evaluation.
-__device__ __forceinline__ void wl_push(const StepParams& p, int e, int wf) {
-    if (wf & WL_TRIGGER) p.wl[atomicAdd(p.wl_count, 1)] = make_int2(e, wf);
+// with one late-started evaluation.  Flush-only entries (most entries) go to a list of their own, which the post kernel
+// works through in units of 32 vehicles per warp after the other entries; they carry the env's k_done and k_now, so the
+// post kernel never reads env4 of an env whose k_done another warp of the same launch may already have advanced.
+__device__ __forceinline__ void wl_push(const StepParams& p, int e, int wf, int k_done, int k_now) {
+    if (wf == WL_FLUSH) p.wl_flush[atomicAdd(p.wl_count + 3, 1)] = make_int4(e, k_done, k_now, 0);
+    else if (wf & WL_TRIGGER) p.wl[atomicAdd(p.wl_count, 1)] = make_int2(e, wf);
     else p.wl[p.E - 1 - atomicAdd(p.wl_count + 2, 1)] = make_int2(e, wf);
 }
 __device__ __forceinline__ int2 wl_fetch(const StepParams& p, int w, int n_front) {
@@ -1161,7 +1170,7 @@ __global__ void __launch_bounds__(kThreads, kMinCtasPerSm) fleet_step_kernel(con
             p.env_f64[(size_t)EF_EP_RETURN * p.E + e] = ep_ret;
             st_keep_v4(p.env4 + e, make_int4(es.t + 1, es.t_start, es.ep_count, es.k_done), keep);
             const int wf = wl_flags(p, es.flags, es.t - es.t_start, es.k_done);
-            if (wf) wl_push(p, e, wf);   // the post kernel evaluates the degradation first and resets afterwards, like the reference
+            if (wf) wl_push(p, e, wf, es.k_done, es.t + 1 - es.t_start);   // the post kernel evaluates the degradation first and resets afterwards, like the reference
         }
         p.env_f64[(size_t)EF_REWARD64 * p.E + e] = reward;
         p.env_f64[(size_t)EF_CASHFLOW * p.E + e] = cashflow;
@@ -1568,7 +1577,7 @@ __global__ void __launch_bounds__(pf_threads(kV)) __maxnreg__(pf_maxreg(kV)) fle
                 p.env_f64[(size_t)EF_EP_RETURN * p.E + e] = ep_ret;
                 st_keep_v4(p.env4 + e, make_int4(es.t + 1, es.t_start, es.ep_count, es.k_done), keep);
                 const int wf = wl_flags(p, es.flags, es.t - es.t_start, es.k_done);
-                if (wf) wl_push(p, e, wf);
+                if (wf) wl_push(p, e, wf, es.k_done, es.t + 1 - es.t_start);
                 p.env_f64[(size_t)EF_REWARD64 * p.E + e] = reward;
                 p.env_f64[(size_t)EF_CASHFLOW * p.E + e] = cashflow;
                 p.env_f64[(size_t)EF_OVERLOAD * p.E + e] = overload;
@@ -1862,12 +1871,17 @@ __global__ void __launch_bounds__(pf_threads(kV)) __maxnreg__(pf_maxreg(kV)) fle
 //   WL_FLUSH    is about to wrap its history ring: consume the pending samples (no evaluation);
 //   WL_RESET    finished its episode with auto-reset on: FleetEnv.reset (:330-434) AFTER the evaluation, i.e. the order in
 //               which a SubprocVecEnv worker runs them.
-// The last CTA of a post kernel to finish clears the work list for the next step.
+// Entries that are WL_FLUSH and nothing else are not work items: once the items are exhausted, every warp consumes them
+// in flush units of 32 vehicles (see the end of fleet_post_kernel).
+// The last CTA of a post kernel to finish clears the work lists for the next step.
 __device__ __forceinline__ void post_finish_lists(const StepParams& p) {
     if (threadIdx.x == 0) {
         __threadfence();
         const unsigned int d = atomicAdd(p.wl_done, 1u);
-        if (d == gridDim.x - 1) { p.wl_count[0] = 0; p.wl_count[1] = 0; p.wl_count[2] = 0; *p.wl_done = 0; }
+        if (d == gridDim.x - 1) {
+            p.wl_count[0] = 0; p.wl_count[1] = 0; p.wl_count[2] = 0; p.wl_count[3] = 0; p.wl_count[4] = 0;
+            *p.wl_done = 0;
+        }
     }
 }
 
@@ -1921,7 +1935,7 @@ __global__ void __launch_bounds__(kT, kT == 32 ? 2 * POST_MIN_CTAS : POST_MIN_CT
         PT_COUNT(11, 1);
         if (p.rf_on && (wf & (WL_TRIGGER | WL_FLUSH))) {
             PT_COUNT(12, 1);
-            const double deg = rf_vehicle<kT>(p, e, n, mine, ev.w, k_now, (wf & WL_TRIGGER) != 0, s_temp, sm_stack + tid,
+            const double deg = rf_vehicle<kT, true>(p, e, n, mine, ev.w, k_now, (wf & WL_TRIGGER) != 0, s_temp, sm_stack + tid,
                                               sm_queue + tid, sm_pend + tid);             // (all lanes of a warp go in together)
             if (deg != 0) atomicAdd(&s_deg, deg);
         } else if ((wf & WL_TRIGGER) && mine) {         // EmpiricalDegradation: the last two samples only
@@ -1966,6 +1980,42 @@ __global__ void __launch_bounds__(kT, kT == 32 ? 2 * POST_MIN_CTAS : POST_MIN_CT
         PT_MARK(9);
         if (tid == 0) { s_w = w_next; s_ent = ent_next; s_ev = ev_next; s_deg = 0; }
     }
+
+    // Flush units: the flush-only entries as one flattened index space of (entry, vehicle) pairs, cut into units of 32
+    // consecutive vehicles.  Each warp fetches units on its own (no CTA barrier), lane l takes vehicle 32 u + l, so a unit
+    // may span two or more envs; a flush needs no evaluation, no reset and no shared sum.  Whoever holds vehicle N-1 of an
+    // env stores its new k_done.
+    const int n_flush = p.wl_count[3];
+    if (n_flush > 0) {
+        const unsigned full = 0xffffffffu;
+        const int lane = tid & 31;
+        const int vehicles = n_flush * N;                // < 2^31: E * N is checked at create time
+        const int units = (vehicles + 31) >> 5;
+        for (;;) {
+            int u = 0;
+            if (lane == 0) u = atomicAdd(p.wl_count + 4, 1);
+            u = __shfl_sync(full, u, 0);
+            if (u >= units) break;
+#ifdef POST_TIMING
+            const long long pt_u = clock64();
+#endif
+            const int v = (u << 5) + lane;
+            const bool active = v < vehicles;
+            int4 fe = make_int4(0, 0, 0, 0);             // an inactive lane reads env 0, row 0, and consumes nothing
+            int n = 0;
+            if (active) {
+                const int f = v / N;
+                n = v - f * N;
+                fe = p.wl_flush[f];
+            }
+            if (active && n == N - 1) p.env4[fe.x].w = fe.z;     // samples up to k_now are consumed (read by the next step)
+            rf_vehicle<kT, false>(p, fe.x, n, active, fe.y, fe.z, false, s_temp, sm_stack + tid, sm_queue + tid, sm_pend + tid);
+#ifdef POST_TIMING
+            if (lane == 0) { atomicAdd(&g_post_clk[15], 1ull); atomicAdd(&g_post_clk[0], (unsigned long long)(clock64() - pt_u)); }
+#endif
+        }
+    }
+    __syncthreads();                                     // no warp of this CTA fetches a unit once the lists are cleared
     post_finish_lists(p);
 }
 
@@ -2693,6 +2743,7 @@ int fleet_create(const FleetConsts* consts, const FleetTables* tb, int32_t num_e
     if ((rc = dev_alloc(h, &p.stats, (size_t)kStatStripes * FLEET_S__COUNT))) return rc;
     if ((rc = dev_alloc(h, &p.err_flags, (size_t)4))) return rc;
     if ((rc = dev_alloc(h, &p.wl, (size_t)E))) return rc;
+    if ((rc = dev_alloc(h, &p.wl_flush, (size_t)E))) return rc;
     if (rf_on) {
         if ((rc = dev_alloc(h, &p.rf_stack, EN * (size_t)rfS))) return rc;
         if ((rc = dev_alloc(h, &p.rf_dc, EN))) return rc;
@@ -2702,7 +2753,7 @@ int fleet_create(const FleetConsts* consts, const FleetTables* tb, int32_t num_e
         if ((rc = dev_alloc(h, &p.ext_val, (size_t)(rfP > 0 ? rfP : 1) * (size_t)(rfX > 0 ? rfX : 1), false))) return rc;
         CUDA_TRY(h, cudaMemset(p.ext_owner, 0xff, sizeof(int) * (size_t)(rfP > 0 ? rfP : 1)));
     }
-    if ((rc = dev_alloc(h, &p.wl_count, (size_t)4))) return rc;
+    if ((rc = dev_alloc(h, &p.wl_count, (size_t)8))) return rc;
     if ((rc = dev_alloc(h, &p.wl_done, (size_t)4))) return rc;
 
     p.rf_on = rf_on ? 1 : 0; p.rf_S = rfS; p.rf_X = rfX; p.rf_P = rfP;

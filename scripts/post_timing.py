@@ -1,4 +1,4 @@
-"""Diagnostic: cycles per phase of the post kernel (needs a -DPOST_TIMING build: `make timing`, run with
+"""Diagnostic: cycles per phase of the post kernel and per flush unit (needs a -DPOST_TIMING build: `make timing`, run with
 FLEETSTEP_LIB=fleetrl_b200/libfleetstep_timing.so)."""
 import ctypes as C, os, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
@@ -40,3 +40,5 @@ print(f"entries per step {ent:.0f}, with rainflow work {deg:.0f}, micro-op itera
 print(f"reset entries per step {v[13] / K:.0f}: reset work of thread 0 {v[14] / max(v[13], 1):.0f} cycles per reset entry (mark 8 -> after post_reset_env)")
 for k in range(1, 10):
     print(f"  {names[k]:28s} {v[k] / max(v[11 if k >= 8 else 12], 1):9.0f} cycles per entry")
+print(f"flush units (32 vehicles of flush-only entries per warp) per step {v[15] / K:.0f}: "
+      f"{v[0] / max(v[15], 1):.0f} cycles per unit (lane 0 of each warp, fetch to end)")
