@@ -1,5 +1,5 @@
 """Per-step comparison of a FleetStepHandle with the CPU oracle (oracle/fleet_oracle.c), shared by test_gpu_parity.py
-and test_gpu_pipeline.py.
+and test_gpu_pipeline.py, and the `knobs` fixture of the tests that set the library's diagnostic variables.
 
 Bit-exact (asserted with array_equal): done, time index, hours_left, target flags, SOC / soc_deg (see below), rainflow cycle
 counts / rainflow_length, observations (float32), terminal observations, start indices drawn by the device RNG.
@@ -9,11 +9,29 @@ revenue factor), SOH abs 1e-13, fd_cyc rel 1e-11.
 import zlib
 
 import numpy as np
+import pytest
 import torch
 
 from synth_tables import make_consts, make_tables
 
 EXACT = ["time_idx", "finish_idx", "hours_left", "target_soc", "rf_len", "n_cycles", "ep_count"]
+KNOBS = ("FLEETSTEP_KERNEL", "FLEETSTEP_PF_GRID", "FLEETSTEP_POST_GRID", "FLEETSTEP_RF_RING", "FLEETSTEP_RF_STACK",
+         "FLEETSTEP_RF_EXT", "FLEETSTEP_RF_EXT_SLOTS")
+
+
+@pytest.fixture
+def knobs(monkeypatch):
+    """Start from the default kernel selection and geometry; returns a setter for the diagnostic variables (None: unset)."""
+    for k in KNOBS:
+        monkeypatch.delenv(k, raising=False)
+
+    def set_knobs(**kv):
+        for k, v in kv.items():
+            if v is None:
+                monkeypatch.delenv(k, raising=False)
+            else:
+                monkeypatch.setenv(k, str(v))
+    return set_knobs
 
 
 def make_case(name, n_evs, days=12, use_case="lmd", sph=4, episode_hours=24, two_trips=False, over=None):

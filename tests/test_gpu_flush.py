@@ -15,13 +15,11 @@ import numpy as np
 import pytest
 
 from oracle.oracle import OracleFleet
-from parity_util import make_case, run_vs_oracle
+from parity_util import knobs, make_case, run_vs_oracle  # noqa: F401  (knobs: fixture)
 from test_gpu_state import parse_blob
 
 pytestmark = pytest.mark.gpu
 
-KNOBS = ("FLEETSTEP_KERNEL", "FLEETSTEP_PF_GRID", "FLEETSTEP_POST_GRID", "FLEETSTEP_PF_V", "FLEETSTEP_POST_THREADS",
-         "FLEETSTEP_RF_RING", "FLEETSTEP_RF_STACK", "FLEETSTEP_RF_EXT", "FLEETSTEP_RF_EXT_SLOTS")
 
 # N, CTA size of the post kernel, env count, post grid; "slow": 2-entry inline stacks, so deep stacks live in extension slots
 CASES = {
@@ -33,17 +31,6 @@ CASES = {
                                  env=dict(FLEETSTEP_RF_RING=4, FLEETSTEP_RF_STACK=2, FLEETSTEP_RF_EXT_SLOTS=40000),
                                  slow=True),
 }
-
-
-@pytest.fixture
-def knobs(monkeypatch):
-    for k in KNOBS:
-        monkeypatch.delenv(k, raising=False)
-
-    def set_knobs(**kv):
-        for k, v in kv.items():
-            monkeypatch.setenv(k, str(v))
-    return set_knobs
 
 
 def _straddling_units(n_flush, N):

@@ -30,6 +30,9 @@ CASES = {
     "lmd_9ev_10day_episodes": dict(n_evs=9, days=30, use_case="lmd", E=3, steps=1000, episode_hours=240),
     "lmd_50ev_e36": dict(n_evs=50, days=8, use_case="lmd", E=36, steps=120),
     "ut_10ev_e50": dict(n_evs=10, days=10, use_case="ut", E=50, steps=210, episode_hours=48),
+    # no auxiliary block, with and without normalisation: with the "+log" rows below, every pf kernel instance runs here
+    "lmd_10ev_noaux": dict(n_evs=10, days=12, use_case="lmd", E=48, steps=200, over=dict(aux=0)),
+    "lmd_12ev_norm_noaux": dict(n_evs=12, days=12, use_case="lmd", E=40, steps=200, over=dict(normalize=1, aux=0)),
 }
 
 
@@ -42,13 +45,11 @@ KERNELS = ([(n, "pf") for n in sorted(CASES) if CASES[n]["n_evs"] >= 8 and CASES
            + [(n, "pf+ring4+stack2") for n in ("lmd_50ev", "ct_20ev_two_trips", "lmd_9ev_norm_nocarry")]
            + [(n, "generic+ring8+stack3") for n in ("lmd_300ev", "lmd_7ev", "lmd_1ev", "lmd_5ev_soh09", "lmd_4ev_no_autoreset")]
            + [("lmd_9ev_10day_episodes", "pf+ring16+stack4"), ("lmd_50ev", "pf+ring128+stack64")]
-           # the two-vehicles-per-thread variant of the pf kernel (off by default, FLEETSTEP_PF_V=2) and the two-warp /
-           # one-warp work items of the post kernel
-           + [("lmd_50ev", "pf+v2"), ("ct_20ev_two_trips", "pf+v2+post64"), ("ut_10ev_e50", "pf+v2"), ("lmd_50ev_e36", "pf+post32"),
-              ("lmd_300ev", "generic+post32")]
            # pf rows run the instance without the charge log (the one bench.py and FleetVecEnv use); "+log" rows run the
-           # kLog instances of both vehicle widths; generic rows keep the charge log on throughout
-           + [("lmd_50ev", "pf+log"), ("lmd_50ev", "pf+v2+log"), ("lmd_9ev_norm_nocarry", "pf+log")])
+           # kLog instances (all four normalisation x auxiliary-block combinations, and the ct / ut use cases); generic rows
+           # keep the charge log on throughout
+           + [("lmd_50ev", "pf+log"), ("lmd_9ev_norm_nocarry", "pf+log"), ("lmd_10ev_noaux", "pf+log"),
+              ("lmd_12ev_norm_noaux", "pf+log"), ("ct_20ev_two_trips", "pf+log"), ("ut_10ev_e50", "pf+log")])
 
 
 @pytest.mark.parametrize("name,kernel", KERNELS)
@@ -59,8 +60,7 @@ def test_gpu_vs_oracle(name, kernel, monkeypatch):
         monkeypatch.setenv("FLEETSTEP_RF_EXT_SLOTS", "40000")      # tiny inline stacks: every vehicle may need an extension slot
     else:
         monkeypatch.delenv("FLEETSTEP_RF_EXT_SLOTS", raising=False)
-    for var, key in (("FLEETSTEP_RF_RING", "ring"), ("FLEETSTEP_RF_STACK", "stack"), ("FLEETSTEP_RF_EXT", "ext"),
-                     ("FLEETSTEP_PF_V", "v"), ("FLEETSTEP_POST_THREADS", "post")):
+    for var, key in (("FLEETSTEP_RF_RING", "ring"), ("FLEETSTEP_RF_STACK", "stack"), ("FLEETSTEP_RF_EXT", "ext")):
         val = [t[len(key):] for t in kernel.split("+")[1:] if t.startswith(key)]
         if val:
             monkeypatch.setenv(var, val[0])
@@ -99,8 +99,8 @@ def test_rainflow_stack_capacity_is_loud(monkeypatch):
 
 
 def test_sei_stress_accuracy():
-    """The post kernel's series evaluation of the SEI cycle stress (rainflow_sei_degradation.py:68-79) against extended
-    precision: relative error below 5e-14 over the whole argument range (fd_cyc is stated at rel 1e-12 vs the reference)."""
+    """The post kernel's SEI cycle stress (rainflow_sei_degradation.py:68-79, dod ** kd2 as exp(kd2 * log(dod))) against
+    extended precision: relative error below 5e-14 over the whole argument range (fd_cyc is stated at rel 1e-12 vs the reference)."""
     import ctypes as C
     from fleetrl_b200._lib import load_library
     L = load_library()

@@ -13,28 +13,11 @@ import torch
 
 from golden_util import Golden, golden_names
 from oracle.oracle import OracleFleet
-from parity_util import Outputs, make_case, run_vs_oracle
+from parity_util import Outputs, knobs, make_case, run_vs_oracle  # noqa: F401  (knobs: fixture)
 
 pytestmark = pytest.mark.gpu
 
-KNOBS = ("FLEETSTEP_KERNEL", "FLEETSTEP_PF_GRID", "FLEETSTEP_POST_GRID", "FLEETSTEP_PF_V", "FLEETSTEP_POST_THREADS",
-         "FLEETSTEP_RF_RING", "FLEETSTEP_RF_STACK", "FLEETSTEP_RF_EXT", "FLEETSTEP_RF_EXT_SLOTS")
 MIN_TILES_PER_CTA = 24
-
-
-@pytest.fixture
-def knobs(monkeypatch):
-    """Start from the default kernel selection and geometry; returns a setter for the diagnostic variables."""
-    for k in KNOBS:
-        monkeypatch.delenv(k, raising=False)
-
-    def set_knobs(**kv):
-        for k, v in kv.items():
-            if v is None:
-                monkeypatch.delenv(k, raising=False)
-            else:
-                monkeypatch.setenv(k, str(v))
-    return set_knobs
 
 
 def _handle(consts, tables, E, env_id_offset=0):
@@ -74,7 +57,7 @@ PIPE = {
     "n50_cfg2_shape_g5": dict(n_evs=50, days=8, G=5),
     "n50_cfg2_shape_g1": dict(n_evs=50, days=8, G=1),
     "n50_cfg2_shape_g1_charge_log": dict(n_evs=50, days=8, G=1, charge_log=True),
-    "n50_v2_g2": dict(n_evs=50, days=8, G=2, env=dict(FLEETSTEP_PF_V=2)),
+    "n12_norm_noaux_g2_charge_log": dict(n_evs=12, G=2, over=dict(normalize=1, aux=0), charge_log=True),
     "n9_norm_nocarry_g3_post1": dict(n_evs=9, G=3, post=1, over=dict(normalize=1, carry_degradation_state=0)),
     "n129_g2_post1": dict(n_evs=129, days=6, G=2, post=1),
     "n129_g2_post2": dict(n_evs=129, days=6, G=2, post=2),

@@ -14,29 +14,12 @@ import torch
 from fleetrl_b200._abi import FIELDS
 from oracle import policies as opol
 from oracle.oracle import OracleFleet
-from parity_util import Outputs, make_case, run_vs_oracle
+from parity_util import Outputs, knobs, make_case, run_vs_oracle  # noqa: F401  (knobs: fixture)
 
 pytestmark = pytest.mark.gpu
 
-KNOBS = ("FLEETSTEP_KERNEL", "FLEETSTEP_PF_GRID", "FLEETSTEP_POST_GRID", "FLEETSTEP_PF_V", "FLEETSTEP_POST_THREADS",
-         "FLEETSTEP_RF_RING", "FLEETSTEP_RF_STACK", "FLEETSTEP_RF_EXT", "FLEETSTEP_RF_EXT_SLOTS")
 MIN_TILES_PER_CTA = 24
 FLIP = 0.9
-
-
-@pytest.fixture
-def knobs(monkeypatch):
-    """Start from the default kernel selection and geometry; returns a setter for the diagnostic variables."""
-    for k in KNOBS:
-        monkeypatch.delenv(k, raising=False)
-
-    def set_knobs(**kv):
-        for k, v in kv.items():
-            if v is None:
-                monkeypatch.delenv(k, raising=False)
-            else:
-                monkeypatch.setenv(k, str(v))
-    return set_knobs
 
 
 def _handle(consts, tables, E, env_id_offset=1000):
@@ -52,9 +35,9 @@ def _capped_envs(consts, tables, G):
     return MIN_TILES_PER_CTA * G * B + (B // 3 + 1 if B > 1 else 1)
 
 
-def _assert_pf_capped(gpu, G, kV=1):
+def _assert_pf_capped(gpu, G):
     g = gpu.launch_geometry
-    assert gpu.step_kernel_name == f"fleet_step_pf_kernel<kV={kV}>", gpu.step_kernel_name
+    assert gpu.step_kernel_name == "fleet_step_pf_kernel<kV=1>", gpu.step_kernel_name
     assert g["step_grid"] == G and g["step_tiles"] // G >= MIN_TILES_PER_CTA, g
     return g
 
@@ -100,7 +83,7 @@ def parse_blob(blob):
 # evaluation within the first two simulated days (SEI: 6.5e-5 per day at most, linear: 3.4e-6).
 FLIP_CASES = {
     "pf_v1_g2": dict(n_evs=8, G=2, delta=3e-5, policies=True),
-    "pf_v2_linear_g1": dict(n_evs=10, G=1, delta=2e-6, kV=2, over=dict(deg_mode=1), env=dict(FLEETSTEP_PF_V=2)),
+    "pf_linear_g1": dict(n_evs=10, G=1, delta=2e-6, over=dict(deg_mode=1)),
     "generic_n7": dict(n_evs=7, E=150, delta=3e-5, policies=True),
     "pf_norm_aux_g1": dict(n_evs=13, G=1, delta=3e-5, over=dict(normalize=1)),
     "pf_ct_two_trips_g1": dict(n_evs=12, G=1, delta=3e-5, use_case="ct", two_trips=True, policies=True),
@@ -120,8 +103,8 @@ def _soh_writes(E, N, lo=FLIP - 2e-9, hi=FLIP + 2e-9):
 
 
 class FlipWatch:
-    """Scenario counters of a flip run: tiles with flipped and unflipped vehicles, two vehicles of one kV=2 thread that
-    differ, flips of vehicles whose SOH was not written, envs whose flags a reset cleared while others stay set, and
+    """Scenario counters of a flip run: tiles with flipped and unflipped vehicles, two vehicles of one lane pair (even N:
+    vehicles 2m and 2m+1 of an env, whose contributions the pf kernel pre-adds with a shuffle) that differ, flips of vehicles whose SOH was not written, envs whose flags a reset cleared while others stay set, and
     policy actions that the flip changed (on a sample of envs; the device computes all of them)."""
 
     def __init__(self, gpu, orc, consts, tables, B, written, policies):
@@ -176,11 +159,11 @@ class FlipWatch:
 @pytest.mark.parametrize("name", sorted(FLIP_CASES))
 def test_partial_flips_vs_oracle(name, knobs):
     """SOH written just below, at and just above 0.9 for single vehicles after the reset, init_soh just above 0.9:
-    flipped and unflipped vehicles share tiles (and kV=2 threads), the counter goes from 0 to non-zero during the run,
+    flipped and unflipped vehicles share tiles (and lane pairs), the counter goes from 0 to non-zero during the run,
     daily evaluations flip further vehicles later, and (carry_degradation_state=0) resets clear flags while the counter
     stays.  Every output and state field, target_soc included, is compared with the oracle after every step."""
     cf = dict(FLIP_CASES[name])
-    G, kV, delta = cf.pop("G", None), cf.pop("kV", 1), cf.pop("delta")
+    G, delta = cf.pop("G", None), cf.pop("delta")
     policies, E = cf.pop("policies", False), cf.pop("E", None)
     knobs(**cf.pop("env", {}))
     cf["over"] = dict(cf.get("over", {}), init_soh=FLIP + delta)
@@ -194,7 +177,7 @@ def test_partial_flips_vs_oracle(name, knobs):
     if G is None:
         assert gpu.step_kernel_name == "fleet_step_kernel"
     else:
-        _assert_pf_capped(gpu, G, kV)
+        _assert_pf_capped(gpu, G)
     N, L = gpu.N, consts.episode_steps
     orc = OracleFleet(consts, tables, E, env_id_offset=1000, threads=8)
     w = _soh_writes(E, N)
@@ -212,7 +195,7 @@ def test_partial_flips_vs_oracle(name, knobs):
     r = {k: getattr(watch, k) for k in ("mixed_tiles", "mixed_pairs", "late_flips", "cleared", "policy_flip_diffs")}
     assert watch.flips_per_step[0] > 0, r                    # 0 at the reset, > 0 after the first step
     assert r["mixed_tiles"] > 0 and r["late_flips"] > 0, r
-    if kV == 2:
+    if G is not None and N % 2 == 0:
         assert r["mixed_pairs"] > 0, r
     if not consts.carry_degradation_state:
         assert r["cleared"] > 0, r
