@@ -5,7 +5,7 @@ NVCCFLAGS = $(ARCH) -O3 -lineinfo -std=c++17 -fmad=false -Xcompiler -fPIC,-ffp-c
 LIB = fleetrl_b200/libfleetstep.so
 
 all: $(LIB) oracle
-SRCS = fleetrl_b200/csrc/fleetstep.cu fleetrl_b200/csrc/vecnorm.cu
+SRCS = fleetrl_b200/csrc/fleetstep.cu fleetrl_b200/csrc/vecnorm.cu fleetrl_b200/csrc/rollout.cu
 $(LIB): $(SRCS) include/fleetstep.h
 	$(NVCC) $(NVCCFLAGS) -Xptxas -v -shared -o $@ $(SRCS)
 timing:   # diagnostic build with per-phase cycle counters in the post kernel (scripts/post_timing.py)

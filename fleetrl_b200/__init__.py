@@ -13,6 +13,9 @@ def __getattr__(name):  # lazy: importing the package must not require torch / C
     if name == "FleetVecNormalize":
         from . import normalize
         return normalize.FleetVecNormalize
+    if name in ("FleetRolloutBuffer", "RolloutBufferSamples", "collect_rollouts"):
+        from . import rollout
+        return getattr(rollout, name)
     if name in ("build_fleet", "FleetInputs"):
         from . import tables
         return getattr(tables, name)

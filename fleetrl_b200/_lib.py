@@ -26,11 +26,19 @@ EXPORTS = [
     "fleet_launch_geometry",
     "fleet_norm_create", "fleet_norm_destroy", "fleet_norm_set_flags", "fleet_norm_moments_len", "fleet_norm_moments",
     "fleet_norm_apply", "fleet_norm_reset_returns", "fleet_norm_get_state", "fleet_norm_set_state", "fleet_norm_last_error",
+    "fleet_rollout_add", "fleet_rollout_gae", "fleet_rollout_gather", "fleet_rollout_last_error",
 ]
 
 
 class FleetStepError(RuntimeError):
     pass
+
+
+class FleetRolloutBuf(C.Structure):
+    """struct FleetRolloutBuf of fleetstep.h: sizes and the device pointers of a rollout buffer's eight arrays."""
+    _fields_ = [(n, C.c_int32) for n in ("buffer_size", "num_envs", "obs_dim", "action_dim")] + \
+               [(n, C.c_void_p) for n in ("observations", "actions", "rewards", "episode_starts", "values", "log_probs",
+                                          "advantages", "returns")]
 
 
 def load_library(path: str = LIB_PATH):
@@ -93,6 +101,12 @@ def load_library(path: str = LIB_PATH):
     L.fleet_norm_set_state.argtypes = [vp] * 9
     L.fleet_norm_last_error.argtypes = [vp]
     L.fleet_norm_last_error.restype = C.c_char_p
+    rb = C.POINTER(FleetRolloutBuf)
+    L.fleet_rollout_add.argtypes = [rb, i32] + [vp] * 7
+    L.fleet_rollout_gae.argtypes = [rb, f64, f64, vp, vp, vp]
+    L.fleet_rollout_gather.argtypes = [rb, vp, i64] + [vp] * 7
+    L.fleet_rollout_last_error.argtypes = []
+    L.fleet_rollout_last_error.restype = C.c_char_p
     if L.fleet_abi_version() != ABI_VERSION:
         raise FleetStepError("libfleetstep.so ABI version does not match fleetrl_b200/_abi.py")
     _LIB = L

@@ -367,6 +367,53 @@ int fleet_norm_set_state(FleetNorm* n, const double* obs_mean, const double* obs
 
 const char* fleet_norm_last_error(const FleetNorm* n);
 
+/*
+ * FleetRollout — SB3 2.3.2's RolloutBuffer (stable_baselines3/common/buffers.py), the transition storage of PPO, on the
+ * device.  Stateless: the caller owns the storage, [T][E]... float32 arrays described by a FleetRolloutBuf
+ * (T = buffer_size, E = num_envs), laid out like RolloutBuffer's attributes before swap_and_flatten.  One kernel launch per
+ * call, no host synchronisation, no atomics (deterministic).  Offsets are 64-bit.  FLEET_E_INVALID for sizes < 1 or a
+ * NULL storage pointer; fleet_rollout_last_error() returns the message of the calling thread's last failure.
+ */
+typedef struct FleetRolloutBuf {
+    int32_t buffer_size, num_envs, obs_dim, action_dim;
+    float* observations;      /* [T][E][obs_dim]     RolloutBuffer.observations                        */
+    float* actions;           /* [T][E][action_dim]  .actions (unclipped, as the policy sampled them)  */
+    float* rewards;           /* [T][E]              .rewards                                          */
+    float* episode_starts;    /* [T][E]              .episode_starts, 0.0f / 1.0f                      */
+    float* values;            /* [T][E]              .values                                           */
+    float* log_probs;         /* [T][E]              .log_probs                                        */
+    float* advantages;        /* [T][E]              .advantages                                       */
+    float* returns;           /* [T][E]              .returns                                          */
+} FleetRolloutBuf;
+
+/* RolloutBuffer.add (buffers.py) into slot `slot` (its self.pos): obs float32 [E][obs_dim], action [E][action_dim],
+ * reward / value / log_prob float32 [E], episode_start uint8 [E] (the env's done dtype) stored as 0.0f / 1.0f.  Any source
+ * may be NULL, which leaves that field of the slot untouched (an on-device collector writes the reward after the env step
+ * that overwrites the observation).  FLEET_E_INVALID for a slot outside [0, buffer_size).  Views need not be aligned. */
+int fleet_rollout_add(const FleetRolloutBuf* b, int32_t slot, const float* obs, const float* action, const float* reward,
+                      const uint8_t* episode_start, const float* value, const float* log_prob, void* stream);
+
+/* RolloutBuffer.compute_returns_and_advantage (buffers.py) over the whole buffer: last_values float32 [E], dones uint8 [E]
+ * (both required).  SB3's float32 arithmetic in SB3's order, bit for bit, with g = float32(gamma) and
+ * gl = float32(gamma * gae_lambda):
+ *   delta = (rewards[t] + (g * next_values) * nnt) - values[t];   last_gae_lam = delta + (gl * nnt) * last_gae_lam
+ *   advantages[t] = last_gae_lam;   returns[t] = last_gae_lam + values[t]
+ * nnt = 1 - dones at t = T-1, else 1 - episode_starts[t+1].  FLEET_E_INVALID for gamma or gae_lambda outside [0, 1]. */
+int fleet_rollout_gae(const FleetRolloutBuf* b, double gamma, double gae_lambda, const float* last_values,
+                      const uint8_t* dones, void* stream);
+
+/* RolloutBuffer._get_samples (buffers.py) for `count` flat sample indices (int64, device).  SB3 numbers the samples after
+ * swap_and_flatten, env-major: flat k is env k / T, step k % T; this reads row (k % T) * E + k / T of the [T][E] storage,
+ * so the one-off flattened copy SB3 makes in get() is not needed.  Writes obs_out [count][obs_dim],
+ * actions_out [count][action_dim] and values / log_probs / advantages / returns _out [count] (all required).  An index
+ * outside [0, T*E) writes nothing to its output row.  FLEET_E_INVALID for count < 0. */
+int fleet_rollout_gather(const FleetRolloutBuf* b, const int64_t* flat_idx_dev, int64_t count, float* obs_out,
+                         float* actions_out, float* values_out, float* log_probs_out, float* advantages_out,
+                         float* returns_out, void* stream);
+
+/* Message of the calling thread's last failing fleet_rollout_* call. */
+const char* fleet_rollout_last_error(void);
+
 #ifdef __cplusplus
 }
 #endif
