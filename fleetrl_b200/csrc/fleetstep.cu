@@ -5,7 +5,10 @@
 //                 fleet_step_kernel (generic: any N, frozen envs): EvCharger.charge + LoadCalculation.check_violation +
 //                 ScoreConfig penalties + time advance + departure/arrival logic + Observer/Normalization observation
 //                 assembly for E envs x N EVs; appends the new soc_deg sample to a small per-env ring and pushes envs that
-//                 need more onto a device work list.
+//                 need more onto a device work list.  The two kernels share the per-vehicle step (ev_slot_step) and
+//                 the env-level parts (stage_env_scratch, obs_row_dst, finalise_env); they differ in how inputs are
+//                 fetched, how the per-env sums are reduced, how the observation tile is stored and in launch
+//                 geometry.
 //   post kernel   fleet_post_kernel: incremental rainflow (persistent three-point stack per vehicle) over the ring samples,
 //                 at the daily 14:45 trigger RainflowSeiDegradation / EmpiricalDegradation.calculate_degradation, then the
 //                 SB3-style auto-reset of finished envs.
@@ -160,11 +163,10 @@ struct StepParams {
 
 enum { EF_EP_RETURN = 0, EF_LAST_EP_RETURN, EF_REWARD64, EF_CASHFLOW, EF_OVERLOAD, EF_SOC_VIOL, EF__COUNT };
 
-struct EnvS {  // per-env scratch of a tile, shared memory
+struct EnvS {  // per-env scratch of a tile, shared memory (both step kernels; stage_env_scratch fills it)
     int t, t_start, ep_count, flags;
     double S, F_cr, F_dr, Rfac, pv_share, gml, pvv;
-    float* obs_dst;
-    int k_done;
+    int k_done, pad;
 };
 
 __device__ __forceinline__ unsigned long long mix64(unsigned long long z) {
@@ -181,6 +183,16 @@ __device__ __forceinline__ int draw_start(unsigned long long seed, int start_lo,
         mix64(seed ^ mix64((unsigned long long)env_id * 0xD1B54A32D192ED03ull + (unsigned long long)(unsigned)episode_no));
     unsigned long long span = (unsigned long long)(start_hi - start_lo) + 1ull;
     return start_lo + (int)(h % span);
+}
+// Start index of env e's next episode: starts[e] when the caller supplies start indices, else the draw for episode
+// ep_count (the number of episodes the env has begun so far).
+__device__ __forceinline__ int episode_start(const StepParams& p, const int* starts, int e, int ep_count) {
+    return starts ? starts[e] : draw_start(p.seed, p.start_lo, p.start_hi, p.env_id_offset + e, ep_count);
+}
+// env4 and episode return of env e when its next episode begins at time index t0.
+__device__ __forceinline__ void begin_episode(const StepParams& p, int e, int t0, int ep_count) {
+    p.env4[e] = make_int4(t0, t0, ep_count + 1, 0);
+    p.env_f64[(size_t)EF_EP_RETURN * p.E + e] = 0;
 }
 
 
@@ -208,24 +220,8 @@ __device__ __forceinline__ void st_keep_v4(void* ptr, int4 v, uint64_t pol) {
                  :: "l"(ptr), "r"(v.x), "r"(v.y), "r"(v.z), "r"(v.w), "l"(pol) : "memory");
 }
 
-__device__ __forceinline__ EvRec load_rec(const EvRec* ptr) {
-    // two 128-bit read-only loads of one 32-byte sector (tables keep the default L2 policy; streaming state uses
-    // evict-first loads/stores so the tables stay resident)
-    const int4 v = __ldg(reinterpret_cast<const int4*>(ptr));
-    const float4 w = __ldg(reinterpret_cast<const float4*>(ptr) + 1);
-    EvRec r;
-    r.sr = __hiloint2double(v.y, v.x);
-    r.tl = __int_as_float(v.z);
-    r.there = (uint8_t)(v.w & 0xff);
-    r.there_prev = (uint8_t)((v.w >> 8) & 0xff);
-    r.pad = 0;
-    r.tt = w.x; r.cl = w.y; r.hn = w.z; r.lax = w.w;
-    return r;
-}
-
-__device__ __forceinline__ EvRec load_rec_keep(const EvRec* ptr, uint64_t pol) {
-    const int4 v = ld_keep_v4(ptr, pol);
-    const int4 w = ld_keep_v4(reinterpret_cast<const int4*>(ptr) + 1, pol);
+// An EvRec from the two 128-bit halves of its 32-byte sector.
+__device__ __forceinline__ EvRec decode_rec(int4 v, int4 w) {
     EvRec r;
     r.sr = __hiloint2double(v.y, v.x);
     r.tl = __int_as_float(v.z);
@@ -234,6 +230,16 @@ __device__ __forceinline__ EvRec load_rec_keep(const EvRec* ptr, uint64_t pol) {
     r.pad = 0;
     r.tt = __int_as_float(w.x); r.cl = __int_as_float(w.y); r.hn = __int_as_float(w.z); r.lax = __int_as_float(w.w);
     return r;
+}
+
+__device__ __forceinline__ EvRec load_rec(const EvRec* ptr) {
+    // two 128-bit read-only loads of one 32-byte sector (tables keep the default L2 policy; streaming state uses
+    // evict-first loads/stores so the tables stay resident)
+    return decode_rec(__ldg(reinterpret_cast<const int4*>(ptr)), __ldg(reinterpret_cast<const int4*>(ptr) + 1));
+}
+
+__device__ __forceinline__ EvRec load_rec_keep(const EvRec* ptr, uint64_t pol) {
+    return decode_rec(ld_keep_v4(ptr, pol), ld_keep_v4(reinterpret_cast<const int4*>(ptr) + 1, pol));
 }
 
 // Auxiliary observation terms for a vehicle whose target SOC was raised to 0.9 (rare; the table holds the values
@@ -272,14 +278,18 @@ __device__ __forceinline__ void write_ev_obs(const StepParams& p, float* __restr
 }
 
 // Time-only part of the observation (price/tariff/load/pv windows, evse/grid terms, calendar sin/cos): a host-
-// precomputed float32 row per time index, copied by the env's slot threads.
+// precomputed float32 row of Ha + Hb elements per time index.  Element q of it goes to position hdr_pos(q) of the
+// observation row: the first Ha after the per-EV soc / hours_left, the Hb others (aux only) after the auxiliary block.
+template <bool kAux>
+__device__ __forceinline__ int hdr_pos(int Ha, int N, int q) {
+    return q < Ha ? 2 * N + q : 2 * N + Ha + (kAux ? 5 * N : 0) + (q - Ha);
+}
+// The header row of time t, copied by the env's slot threads.  Without aux Hb is 0 and the bound is written as Ha: as a
+// compile-time choice it keeps fleet_reset_kernel one register lower.
 template <bool kAux>
 __device__ __forceinline__ void copy_hdr(const StepParams& p, float* __restrict__ o, int n, int t) {
     const float* __restrict__ h = p.hdr + (size_t)t * p.hdr_stride;
-    const int N = p.N;
-    for (int q = n; q < p.Ha; q += N) o[2 * N + q] = __ldg(h + q);
-    if (kAux)
-        for (int q = n; q < p.Hb; q += N) o[2 * N + p.Ha + 5 * N + q] = __ldg(h + p.Ha + q);
+    for (int q = n; q < (kAux ? p.Ha + p.Hb : p.Ha); q += p.N) o[hdr_pos<kAux>(p.Ha, p.N, q)] = __ldg(h + q);
 }
 
 // FleetEnv.reset for one (env, EV) slot: fleet_environment.py:345-348, 371-372, 382-399.
@@ -790,8 +800,7 @@ __device__ __forceinline__ void bulk_store_wait_read() {
 //   in : es (per-env factors of time t: S, F_cr, F_dr, Rfac, pv_share, flags), a = action, soh, sr / ntl = schedule
 //        SOC_on_return / time_left at t+1, there = presence at t, flip = target already raised to 0.9
 //   io : soc, hl, sdeg      out: the vehicle's terms of the five per-env sums
-template <class EnvT>
-__device__ __forceinline__ void ev_slot_step(const StepParams& p, const EnvT& es, size_t i, bool flip, double a, double soh,
+__device__ __forceinline__ void ev_slot_step(const StepParams& p, const EnvS& es, size_t i, bool flip, double a, double soh,
                                              double sr, float ntl, int there, double& soc, float& hl, double& sdeg,
                                              double& q_rew, double& q_cash, double& q_ath, double& q_miss, double& q_nviol,
                                              double& q_en) {
@@ -886,6 +895,87 @@ __device__ __forceinline__ int wl_flags(const StepParams& p, int env_flags, int 
     return wf;
 }
 
+// ---- env-level parts of a step, one thread per env, shared by the two step kernels
+// Fills the env scratch of env4 = {t, t_start, ep_count, k_done} from env4 and the four 128-bit words r0..r3 of
+// step_row[min(t, T - 2)], and returns its EF_* flags.  Without auto-reset an env whose episode is over is frozen until
+// the caller resets it; the pf kernel, which only runs with auto-reset, passes auto_reset = true so that this test
+// folds away.
+__device__ __forceinline__ int stage_env_scratch(const StepParams& p, EnvS& es, int4 env4, int4 r0, int4 r1, int4 r2,
+                                                 int4 r3, bool auto_reset) {
+    es.t = env4.x; es.t_start = env4.y; es.ep_count = env4.z; es.k_done = env4.w;
+    const int t_fin = env4.y + p.L;
+    const uint32_t fn = (uint32_t)r3.w;                                  // flags_next
+    int fl = 0;
+    if (!auto_reset && env4.x >= t_fin) {
+        fl = EF_FROZEN;
+    } else {
+        if (env4.x + 1 == t_fin) fl |= auto_reset ? EF_DONE | EF_RESET : EF_DONE;
+        if ((fn & TF_TRIGGER) && p.calc_deg) fl |= EF_TRIGGER;
+        if (fn & TF_LUNCH) fl |= EF_LUNCH;
+    }
+    es.flags = fl;
+    es.S = __hiloint2double(r0.y, r0.x); es.F_cr = __hiloint2double(r0.w, r0.z);
+    es.F_dr = __hiloint2double(r1.y, r1.x); es.Rfac = __hiloint2double(r1.w, r1.z);
+    es.pv_share = __hiloint2double(r2.y, r2.x); es.gml = __hiloint2double(r2.w, r2.z);
+    es.pvv = __hiloint2double(r3.y, r3.x);
+    return fl;
+}
+
+// Where env e's observation row of this step goes, or nullptr when the caller did not ask for that array.  SB3
+// semantics: a finished env returns the first observation of its next episode in obs (written by the post kernel) and
+// the last observation of the finished one in infos["terminal_observation"].
+__device__ __forceinline__ float* obs_row_dst(const StepParams& p, int flags, int e) {
+    float* const base = (flags & EF_RESET) ? p.terminal_obs : p.obs;
+    return base ? base + (size_t)e * p.D : nullptr;
+}
+
+// End of env e's step from its per-env sums sums[q * B + bb]: cashflow, reward with the overload penalty
+// (score_config.py:33-41), soc violation, done, episode return (ep_prev: the return so far), the statistics in stripe
+// st, the advanced env4, the work-list push and the outputs.  A frozen env reports done with zero reward and adds no
+// statistics.
+__device__ __forceinline__ void finalise_env(const StepParams& p, const EnvS& es, int e, const double* sums, int B,
+                                             int bb, double* st, double ep_prev, uint64_t keep) {
+    double reward = 0, cashflow = 0, overload = 0, soc_viol = 0;
+    int done = 0;
+    if (es.flags & EF_FROZEN) {
+        done = 1;
+    } else {
+        cashflow = sums[Q_CASH * B + bb];
+        reward = sums[Q_REWARD * B + bb];
+        const double margin = es.gml - sums[Q_ATH * B + bb] * p.evse + es.pvv;                 // load_calculation.py:93
+        overload = fabs(margin < 0.0 ? margin : 0.0);
+        if (overload > 0) {
+            const double rel = overload / p.grid + 1;                                          // fleet_environment.py:496
+            const double pen = (rel < 1.1) ? 0.0 : -700 / (1 + exp(-15.77350877 * (rel - 1.33298382)));
+            reward += pen * p.pen_ovl;                                                         // score_config.py:33-41
+            atomicAdd(st + FLEET_S_OVERLOAD_KW, overload);
+        }
+        soc_viol = fabs(sums[Q_MISS * B + bb]);                                                // :661
+        const double n_viol = sums[Q_NVIOL * B + bb];
+        done = (es.flags & EF_DONE) ? 1 : 0;                                                   // :627-628
+        const double ep_ret = ep_prev + reward;                                                // :637
+        atomicAdd(st + FLEET_S_STEPS, 1.0);
+        atomicAdd(st + FLEET_S_REWARD, reward);
+        atomicAdd(st + FLEET_S_CASHFLOW, cashflow);
+        if (n_viol > 0) { atomicAdd(st + FLEET_S_SOC_VIOL, soc_viol); atomicAdd(st + FLEET_S_N_VIOL, n_viol); }
+        if (done) {
+            atomicAdd(st + FLEET_S_EPISODES, 1.0);
+            atomicAdd(st + FLEET_S_EP_RETURN, ep_ret);
+            p.env_f64[(size_t)EF_LAST_EP_RETURN * p.E + e] = ep_ret;
+        }
+        p.env_f64[(size_t)EF_EP_RETURN * p.E + e] = ep_ret;
+        st_keep_v4(p.env4 + e, make_int4(es.t + 1, es.t_start, es.ep_count, es.k_done), keep);
+        const int wf = wl_flags(p, es.flags, es.t - es.t_start, es.k_done);
+        if (wf) wl_push(p, e, wf, es.k_done, es.t + 1 - es.t_start);   // the post kernel evaluates the degradation first and resets afterwards, like the reference
+    }
+    p.env_f64[(size_t)EF_REWARD64 * p.E + e] = reward;
+    p.env_f64[(size_t)EF_CASHFLOW * p.E + e] = cashflow;
+    p.env_f64[(size_t)EF_OVERLOAD * p.E + e] = overload;
+    p.env_f64[(size_t)EF_SOC_VIOL * p.E + e] = soc_viol;
+    if (p.reward) p.reward[e] = (float)reward;
+    if (p.done) p.done[e] = (uint8_t)done;
+}
+
 // Shared-memory layout (dynamic): EnvS envs[B] | double contrib[kNQ][slots] | double sums[kNQ][B] |
 //                                 float obs_tile[B][D] (16-byte aligned)
 __host__ __device__ inline size_t align16(size_t x) { return (x + 15) & ~(size_t)15; }
@@ -917,38 +1007,13 @@ __global__ void __launch_bounds__(kThreads, kMinCtasPerSm) fleet_step_kernel(con
     const uint64_t keep = l2_evict_last_policy();
     int my_any = 0;             // bit1: this env finished and auto-resets (its row goes to terminal_obs)
 
-    // ---- P0: one thread per env: time index, per-time factors, flags
+    // ---- P0: one thread per env: env scratch (stage_env_scratch)
     if (tid < nb) {
-        const int e = e0 + tid;
-        const int4 ev = ld_keep_v4(p.env4 + e, keep);
-        EnvS& es = envs[tid];
-        es.t = ev.x; es.t_start = ev.y; es.ep_count = ev.z; es.k_done = ev.w;
-        const int t_fin = ev.y + p.L;
-        int fl = 0;
-        if (!p.auto_reset && ev.x >= t_fin) fl |= EF_FROZEN;   // episode over and not reset by the caller
-        const int t = min(ev.x, p.T - 2);
-        const StepRow* r = p.step_row + t;
-        const int4 ra = ld_keep_v4(reinterpret_cast<const int4*>(r), keep);
-        const int4 rb = ld_keep_v4(reinterpret_cast<const int4*>(r) + 1, keep);
-        const int4 r1 = ld_keep_v4(reinterpret_cast<const int4*>(r) + 2, keep);
-        const int4 r2 = ld_keep_v4(reinterpret_cast<const int4*>(r) + 3, keep);
-        es.S = __hiloint2double(ra.y, ra.x); es.F_cr = __hiloint2double(ra.w, ra.z);
-        es.F_dr = __hiloint2double(rb.y, rb.x); es.Rfac = __hiloint2double(rb.w, rb.z);
-        es.pv_share = __hiloint2double(r1.y, r1.x); es.gml = __hiloint2double(r1.w, r1.z);
-        es.pvv = __hiloint2double(r2.y, r2.x);
-        const uint32_t fn = (uint32_t)r2.w;                                  // flags_next
-        if (!(fl & EF_FROZEN)) {
-            if (ev.x + 1 == t_fin) fl |= EF_DONE;
-            if ((fn & TF_TRIGGER) && p.calc_deg) fl |= EF_TRIGGER;
-            if (fn & TF_LUNCH) fl |= EF_LUNCH;
-            if ((fl & EF_DONE) && p.auto_reset) fl |= EF_RESET;
-        }
-        es.flags = fl;
-        // SB3 semantics: a finished env returns the first observation of its next episode in obs (written by the
-        // post kernel) and the last observation of the finished one in infos["terminal_observation"].
-        if (fl & EF_RESET) es.obs_dst = p.terminal_obs ? p.terminal_obs + (size_t)e * D : nullptr;
-        else es.obs_dst = p.obs ? p.obs + (size_t)e * D : nullptr;
-        if (fl & EF_RESET) my_any = 2;
+        const int4 ev = ld_keep_v4(p.env4 + e0 + tid, keep);
+        const int4* r = reinterpret_cast<const int4*>(p.step_row + min(ev.x, p.T - 2));
+        const int4 r0 = ld_keep_v4(r, keep), r1 = ld_keep_v4(r + 1, keep), r2 = ld_keep_v4(r + 2, keep),
+                   r3 = ld_keep_v4(r + 3, keep);
+        if (stage_env_scratch(p, envs[tid], ev, r0, r1, r2, r3, p.auto_reset != 0) & EF_RESET) my_any = 2;
     }
 
     const bool have_flips = (*p.n_flips != 0);
@@ -989,7 +1054,7 @@ __global__ void __launch_bounds__(kThreads, kMinCtasPerSm) fleet_step_kernel(con
             const EnvS& eh = envs[bb];
             const int th = (eh.flags & EF_FROZEN) ? min(eh.t, p.T - 1) : min(eh.t + 1, p.T - 1);
             hv = ld_keep_f32(p.hdr + (size_t)th * p.hdr_stride + q, keep);
-            hdst = bb * D + (q < p.Ha ? 2 * N + q : 2 * N + p.Ha + (kAux ? 5 * N : 0) + (q - p.Ha));
+            hdst = bb * D + hdr_pos<kAux>(p.Ha, N, q);
         }
 
         // ---- P1b: charge / discharge, transition, per-EV observation parts (into the shared obs tile)
@@ -1023,8 +1088,7 @@ __global__ void __launch_bounds__(kThreads, kMinCtasPerSm) fleet_step_kernel(con
         const int bb = w / H, q = w - bb * H;
         const EnvS& eh = envs[bb];
         const int th = (eh.flags & EF_FROZEN) ? min(eh.t, p.T - 1) : min(eh.t + 1, p.T - 1);
-        obs_tile[bb * D + (q < p.Ha ? 2 * N + q : 2 * N + p.Ha + (kAux ? 5 * N : 0) + (q - p.Ha))] =
-            __ldg(p.hdr + (size_t)th * p.hdr_stride + q);
+        obs_tile[bb * D + hdr_pos<kAux>(p.Ha, N, q)] = __ldg(p.hdr + (size_t)th * p.hdr_stride + q);
     }
     asm volatile("fence.proxy.async.shared::cta;" ::: "memory");   // writers: generic-proxy stores -> async proxy
     __syncthreads();
@@ -1036,7 +1100,7 @@ __global__ void __launch_bounds__(kThreads, kMinCtasPerSm) fleet_step_kernel(con
     } else {
         for (int w = tid; w < nb * D; w += kThreads) {
             const int bb = w / D;
-            float* dst = envs[bb].obs_dst;
+            float* dst = obs_row_dst(p, envs[bb].flags, e0 + bb);
             if (dst) dst[w - bb * D] = obs_tile[w];
         }
     }
@@ -1052,68 +1116,31 @@ __global__ void __launch_bounds__(kThreads, kMinCtasPerSm) fleet_step_kernel(con
     }
     __syncthreads();
 
-    // ---- P3: one thread per env: cashflow, reward, overload penalty, done, statistics, work list
+    // ---- P3: one thread per env: finalise_env
     if (tid < nb) {
-        const int bb = tid, e = e0 + bb;
-        const EnvS& es = envs[bb];
-        double reward = 0, cashflow = 0, overload = 0, soc_viol = 0;
-        int done = 0;
-        double* st = p.stats + (size_t)(blockIdx.x % kStatStripes) * FLEET_S__COUNT;
-        if (es.flags & EF_FROZEN) {
-            done = 1;
-        } else {
-            cashflow = sums[Q_CASH * B + bb];
-            reward = sums[Q_REWARD * B + bb];
-            const double margin = es.gml - sums[Q_ATH * B + bb] * p.evse + es.pvv;             // load_calculation.py:93
-            overload = fabs(margin < 0.0 ? margin : 0.0);
-            if (overload > 0) {
-                const double rel = overload / p.grid + 1;                                      // fleet_environment.py:496
-                const double pen = (rel < 1.1) ? 0.0 : -700 / (1 + exp(-15.77350877 * (rel - 1.33298382)));
-                reward += pen * p.pen_ovl;                                                     // score_config.py:33-41
-                atomicAdd(st + FLEET_S_OVERLOAD_KW, overload);
-            }
-            soc_viol = fabs(sums[Q_MISS * B + bb]);                                            // :661
-            const double n_viol = sums[Q_NVIOL * B + bb];
-            done = (es.flags & EF_DONE) ? 1 : 0;                                               // :627-628
-            const double ep_ret = p.env_f64[(size_t)EF_EP_RETURN * p.E + e] + reward;          // :637
-            atomicAdd(st + FLEET_S_STEPS, 1.0);
-            atomicAdd(st + FLEET_S_REWARD, reward);
-            atomicAdd(st + FLEET_S_CASHFLOW, cashflow);
-            if (n_viol > 0) { atomicAdd(st + FLEET_S_SOC_VIOL, soc_viol); atomicAdd(st + FLEET_S_N_VIOL, n_viol); }
-            if (done) {
-                atomicAdd(st + FLEET_S_EPISODES, 1.0);
-                atomicAdd(st + FLEET_S_EP_RETURN, ep_ret);
-                p.env_f64[(size_t)EF_LAST_EP_RETURN * p.E + e] = ep_ret;
-            }
-            p.env_f64[(size_t)EF_EP_RETURN * p.E + e] = ep_ret;
-            st_keep_v4(p.env4 + e, make_int4(es.t + 1, es.t_start, es.ep_count, es.k_done), keep);
-            const int wf = wl_flags(p, es.flags, es.t - es.t_start, es.k_done);
-            if (wf) wl_push(p, e, wf, es.k_done, es.t + 1 - es.t_start);   // the post kernel evaluates the degradation first and resets afterwards, like the reference
-        }
-        p.env_f64[(size_t)EF_REWARD64 * p.E + e] = reward;
-        p.env_f64[(size_t)EF_CASHFLOW * p.E + e] = cashflow;
-        p.env_f64[(size_t)EF_OVERLOAD * p.E + e] = overload;
-        p.env_f64[(size_t)EF_SOC_VIOL * p.E + e] = soc_viol;
-        if (p.reward) p.reward[e] = (float)reward;
-        if (p.done) p.done[e] = (uint8_t)done;
+        const int e = e0 + tid;
+        finalise_env(p, envs[tid], e, sums, B, tid, p.stats + (size_t)(blockIdx.x % kStatStripes) * FLEET_S__COUNT,
+                     p.env_f64[(size_t)EF_EP_RETURN * p.E + e], keep);
     }
     if (use_bulk && tid == 0) bulk_store_wait_read();   // the tile must stay valid until the bulk copy has read it
 }
 
 // ------------------------------------------------------------------------------ persistent prefetching step kernel
-// Same arithmetic as fleet_step_kernel.  The generic kernel is bound by exposed memory latency: ~57 % of the
-// scheduler cycles have no eligible warp (ncu), because every warp first waits two dependent round trips
-// (env4 -> schedule record / history row) and the 64-register budget caps residency at 32 warps per SM.  Here
+// Same arithmetic as fleet_step_kernel, through the same functions: ev_slot_step per vehicle, stage_env_scratch,
+// obs_row_dst and finalise_env per env.  What differs is how the work is fed and laid out.  The generic kernel is bound
+// by exposed memory latency: ~57 % of the scheduler cycles have no eligible warp (ncu), because every warp first waits
+// two dependent round trips (env4 -> schedule record / history row) and the 64-register budget caps residency at 32
+// warps per SM.  Here
 //  * CTAs are persistent (grid = #SMs x resident CTAs, 2 per SM) and loop over tiles of B = kPfSlots / N consecutive envs;
 //  * 8 COMPUTE warps, one thread per (env, EV) slot: each thread copies its own inputs of a tile (action, state,
 //    history row, schedule record, header element) into a shared-memory stage with cp.async (LDGSTS) kPfStages tiles
 //    ahead; the per-env time index those addresses depend on is loaded one tile period before the copies are issued,
 //    so that no dependent address ever waits; the slot -> (env, EV) mapping and parameter loads are paid once; with an
 //    even N the two vehicles of a lane pair (same env) pre-add their contributions with one shuffle;
-//  * 2 EPILOGUE warps, behind the compute warps: warp 0 stages the per-env factors (env4, step_row) three tiles ahead
-//    and does the env-level finalisation (reward, overload, statistics, env4, work list); warp 1 sends the finished
-//    observation tile to HBM with TMA bulk stores (cp.async.bulk, SASS UBLKCP) and does the per-env sums (one lane per
-//    (quantity, env), car order), which it hands to warp 0;
+//  * 2 EPILOGUE warps, behind the compute warps: warp 0 loads env4 and step_row and stages the env scratch three tiles
+//    ahead, then runs finalise_env for the current tile, one lane per env (a tile holds at most 32); warp 1 sends the
+//    finished observation tile to HBM with TMA bulk stores (cp.async.bulk, SASS UBLKCP) and does the per-env sums (one
+//    lane per (quantity, env), car order), which it hands to warp 0;
 //  * no CTA-wide barrier in the loop: producer/consumer hand-offs are mbarriers on kPfOut contribution + observation
 //    buffers, kPfEnvs env-scratch buffers and two sums buffers.
 // Selected when auto_reset is on and 8 <= N <= 256 (one pass per tile); otherwise the generic kernel runs.
@@ -1122,12 +1149,6 @@ constexpr int kPfThreads = kPfSlots + 64;      // + two epilogue warps
 // measured on B200 at cfg2: 2 CTAs/SM x 10 warps with ~100 registers (no spills, L1 left for the tables) beat 3 CTAs/SM
 // at 64 registers by 5-6 %
 constexpr int kPfMaxReg = 96;
-
-struct PfEnv {   // per-env scratch of a tile (shared memory, kPfEnvs buffers)
-    int t, t_start, ep_count, flags;
-    double S, F_cr, F_dr, Rfac, pv_share, gml, pvv;
-    int k_done, pad;
-};
 
 // input stage of the pf kernel: the per-slot inputs of one tile, structure of arrays indexed by the slot's thread
 // (byte offsets)
@@ -1140,7 +1161,7 @@ constexpr int kPfEnvs = 4;    // env-scratch buffers: staged three tiles ahead
 // Even N: neighbouring vehicles' contributions are added in the compute warp (one shuffle), halving the buffer.
 __host__ __device__ inline int pf_contrib_slots(int B, int N) { return (N & 1) ? B * N : (B * N) / 2; }
 __host__ __device__ inline size_t pf_smem_bytes(int B, int N, int D) {
-    return align16(kPfEnvs * align16((size_t)B * sizeof(PfEnv)) + kPfOut * align16((size_t)kNQ * pf_contrib_slots(B, N) * 8) +
+    return align16(kPfEnvs * align16((size_t)B * sizeof(EnvS)) + kPfOut * align16((size_t)kNQ * pf_contrib_slots(B, N) * 8) +
                    2 * align16((size_t)kNQ * B * 8) + kPfOut * align16((size_t)B * D * 4 + 12)) + (size_t)kPfStages * kPfStageBytes;
 }
 
@@ -1233,7 +1254,7 @@ __global__ void __maxnreg__(kPfMaxReg) fleet_step_pf_kernel(const StepParams p) 
         PF_START();
         for (int tile = tile0; tile < ntiles; tile += G, it++) {
             const int buf = it % kPfOut, sbuf = it & 1;
-            const PfEnv* envs = reinterpret_cast<const PfEnv*>(envs0 + (it % kPfEnvs) * p.pf_envs_b);
+            const EnvS* envs = reinterpret_cast<const EnvS*>(envs0 + (it % kPfEnvs) * p.pf_envs_b);
             const double* contrib = reinterpret_cast<const double*>(contrib0 + buf * p.pf_contrib_b);
             // the tile sits in shared memory at the 16-byte phase of its destination obs + e0 * D (0 when B * D % 4 == 0)
             const float* obs_tile = reinterpret_cast<const float*>(obs0 + buf * p.pf_obs_b) + (int)(((size_t)tile * (size_t)(B * D)) & 3);
@@ -1255,17 +1276,13 @@ __global__ void __maxnreg__(kPfMaxReg) fleet_step_pf_kernel(const StepParams p) 
                 // rows of finishing envs go to terminal_obs: one bulk store per env row (row e has the same 16-byte phase
                 // in obs, in terminal_obs and in the tile)
                 if (lane < nb) {
-                    const int e = e0 + lane;
-                    float* dst = (envs[lane].flags & EF_RESET) ? (p.terminal_obs ? p.terminal_obs + (size_t)e * D : nullptr)
-                                                               : (p.obs ? p.obs + (size_t)e * D : nullptr);
+                    float* dst = obs_row_dst(p, envs[lane].flags, e0 + lane);
                     if (dst) thread_store_range(dst, obs_tile + (size_t)lane * D, D);
                 }
             } else {
                 for (int w = lane; w < nb * D; w += 32) {
                     const int bb = w / D;
-                    const int e = e0 + bb;
-                    float* dst = (envs[bb].flags & EF_RESET) ? (p.terminal_obs ? p.terminal_obs + (size_t)e * D : nullptr)
-                                                             : (p.obs ? p.obs + (size_t)e * D : nullptr);
+                    float* dst = obs_row_dst(p, envs[bb].flags, e0 + bb);
                     if (dst) dst[w - bb * D] = obs_tile[w];
                 }
             }
@@ -1321,16 +1338,8 @@ __global__ void __maxnreg__(kPfMaxReg) fleet_step_pf_kernel(const StepParams p) 
             const int e = tile * B + lane;
             int fl = 0;
             if (lane < B && tile < ntiles && e < p.E) {
-                PfEnv& es = reinterpret_cast<PfEnv*>(envs0 + ebuf * p.pf_envs_b)[lane];
-                es.t = envA.x; es.t_start = envA.y; es.ep_count = envA.z; es.k_done = envA.w;
-                if (envA.x + 1 == envA.y + p.L) fl |= EF_DONE | EF_RESET;
-                if (((uint32_t)r3.w & TF_TRIGGER) && p.calc_deg) fl |= EF_TRIGGER;
-                if ((uint32_t)r3.w & TF_LUNCH) fl |= EF_LUNCH;
-                es.flags = fl;
-                es.S = __hiloint2double(r0.y, r0.x); es.F_cr = __hiloint2double(r0.w, r0.z);
-                es.F_dr = __hiloint2double(r1.y, r1.x); es.Rfac = __hiloint2double(r1.w, r1.z);
-                es.pv_share = __hiloint2double(r2.y, r2.x); es.gml = __hiloint2double(r2.w, r2.z);
-                es.pvv = __hiloint2double(r3.y, r3.x);
+                EnvS& es = reinterpret_cast<EnvS*>(envs0 + ebuf * p.pf_envs_b)[lane];
+                fl = stage_env_scratch(p, es, envA, r0, r1, r2, r3, true);
             }
             const bool any = __any_sync(0xffffffffu, (fl & EF_RESET) != 0);
             if (lane == 0) s_any_reset[ebuf] = any;
@@ -1349,7 +1358,7 @@ __global__ void __maxnreg__(kPfMaxReg) fleet_step_pf_kernel(const StepParams p) 
         int it = 0;
         for (int tile = tile0; tile < ntiles; tile += G, it++) {
             const int sbuf = it & 1;
-            const PfEnv* envs = reinterpret_cast<const PfEnv*>(envs0 + (it % kPfEnvs) * p.pf_envs_b);
+            const EnvS* envs = reinterpret_cast<const EnvS*>(envs0 + (it % kPfEnvs) * p.pf_envs_b);
             const double* sums_r = sums + sbuf * sums_stride;
             const int e0 = tile * B;
             const int nb = min(B, p.E - e0);
@@ -1367,45 +1376,10 @@ __global__ void __maxnreg__(kPfMaxReg) fleet_step_pf_kernel(const StepParams p) 
             mbar_wait(&bar_sums_ready[sbuf], (uint32_t)((it >> 1) & 1));   // warp 1 has summed tile `tile`
             PF_TRACE(8, it, 1);
 
-            // ---- env-level finalisation: one lane per env
-            for (int bb = lane; bb < nb; bb += 32) {
-                const int e = e0 + bb;
-                const PfEnv& es = envs[bb];
-                double* stt = p.stats + (size_t)(tile % kStatStripes) * FLEET_S__COUNT;
-                const double cashflow = sums_r[Q_CASH * B + bb];
-                double reward = sums_r[Q_REWARD * B + bb];
-                const double margin = es.gml - sums_r[Q_ATH * B + bb] * p.evse + es.pvv;             // load_calculation.py:93
-                const double overload = fabs(margin < 0.0 ? margin : 0.0);
-                if (overload > 0) {
-                    const double rel = overload / p.grid + 1;                                      // fleet_environment.py:496
-                    const double pen = (rel < 1.1) ? 0.0 : -700 / (1 + exp(-15.77350877 * (rel - 1.33298382)));
-                    reward += pen * p.pen_ovl;                                                     // score_config.py:33-41
-                    atomicAdd(stt + FLEET_S_OVERLOAD_KW, overload);
-                }
-                const double soc_viol = fabs(sums_r[Q_MISS * B + bb]);
-                const double n_viol = sums_r[Q_NVIOL * B + bb];
-                const int dn = (es.flags & EF_DONE) ? 1 : 0;
-                const double ep_ret = ((bb == lane) ? ep_prev : p.env_f64[(size_t)EF_EP_RETURN * p.E + e]) + reward;
-                atomicAdd(stt + FLEET_S_STEPS, 1.0);
-                atomicAdd(stt + FLEET_S_REWARD, reward);
-                atomicAdd(stt + FLEET_S_CASHFLOW, cashflow);
-                if (n_viol > 0) { atomicAdd(stt + FLEET_S_SOC_VIOL, soc_viol); atomicAdd(stt + FLEET_S_N_VIOL, n_viol); }
-                if (dn) {
-                    atomicAdd(stt + FLEET_S_EPISODES, 1.0);
-                    atomicAdd(stt + FLEET_S_EP_RETURN, ep_ret);
-                    p.env_f64[(size_t)EF_LAST_EP_RETURN * p.E + e] = ep_ret;
-                }
-                p.env_f64[(size_t)EF_EP_RETURN * p.E + e] = ep_ret;
-                st_keep_v4(p.env4 + e, make_int4(es.t + 1, es.t_start, es.ep_count, es.k_done), keep);
-                const int wf = wl_flags(p, es.flags, es.t - es.t_start, es.k_done);
-                if (wf) wl_push(p, e, wf, es.k_done, es.t + 1 - es.t_start);
-                p.env_f64[(size_t)EF_REWARD64 * p.E + e] = reward;
-                p.env_f64[(size_t)EF_CASHFLOW * p.E + e] = cashflow;
-                p.env_f64[(size_t)EF_OVERLOAD * p.E + e] = overload;
-                p.env_f64[(size_t)EF_SOC_VIOL * p.E + e] = soc_viol;
-                if (p.reward) p.reward[e] = (float)reward;
-                if (p.done) p.done[e] = (uint8_t)dn;
-            }
+            // ---- env-level finalisation: one lane per env (a tile holds at most 32 envs)
+            if (lane < nb)
+                finalise_env(p, envs[lane], e0 + lane, sums_r, B, lane,
+                             p.stats + (size_t)(tile % kStatStripes) * FLEET_S__COUNT, ep_prev, keep);
             __syncwarp();
             if (lane == 0) mbar_arrive(&bar_sums_free[sbuf]);
             PF_TRACE(8, it, 2);
@@ -1419,8 +1393,7 @@ __global__ void __maxnreg__(kPfMaxReg) fleet_step_pf_kernel(const StepParams p) 
     const int b = (N == 1) ? j : (int)__umulhi((unsigned)j, p.n_magic);     // slot -> (env of tile, EV): same for every tile
     const int n = j - b * N;
     const bool slot = j < cstride;
-    auto hdr_pos = [&](int q) { return q < p.Ha ? 2 * N + q : 2 * N + p.Ha + (kAux ? 5 * N : 0) + (q - p.Ha); };
-    const int hpos = hdr_pos(n);
+    const int hpos = hdr_pos<kAux>(p.Ha, N, n);
 
     // Input pipeline: the per-slot inputs of a tile (action, soc, hours_left, soh, previous history row, both halves of
     // ev_rec[t+1], the header element) are copied by the slot's OWN thread into a shared-memory stage with cp.async
@@ -1468,7 +1441,7 @@ __global__ void __maxnreg__(kPfMaxReg) fleet_step_pf_kernel(const StepParams p) 
     PF_DECL();
     PF_START();
     for (int tile = tile0; tile < ntiles; tile += G, it++) {
-        const PfEnv* envs = reinterpret_cast<const PfEnv*>(envs0 + ebuf * p.pf_envs_b);
+        const EnvS* envs = reinterpret_cast<const EnvS*>(envs0 + ebuf * p.pf_envs_b);
         double* contrib = reinterpret_cast<double*>(contrib0 + buf * p.pf_contrib_b);
         float* obs_tile = reinterpret_cast<float*>(obs0 + buf * p.pf_obs_b) + (int)(((size_t)tile * (size_t)(B * D)) & 3);
         const int e0 = tile * B;
@@ -1500,20 +1473,15 @@ __global__ void __maxnreg__(kPfMaxReg) fleet_step_pf_kernel(const StepParams p) 
         float o_hl = 0.f;
         size_t o_hist = 0;
         if (active) {
-            const PfEnv& es = envs[b];
+            const EnvS& es = envs[b];
             float* orow = obs_tile + b * D;
             const size_t i = (size_t)tile * cstride + j;
             const int t1 = min(es.t + 1, p.T - 1);
             const int k = es.t - es.t_start;
             // every input first (the stage and the observation tile may alias as far as the compiler knows: loads placed after
             // the observation stores would have to wait for them)
-            const int4 in_r0 = reinterpret_cast<const int4*>(stp + kPfStR0)[j];
-            const int4 in_r1 = reinterpret_cast<const int4*>(stp + kPfStR1)[j];
-            EvRec rec;
-            rec.sr = __hiloint2double(in_r0.y, in_r0.x); rec.tl = __int_as_float(in_r0.z);
-            rec.there = (uint8_t)(in_r0.w & 0xff); rec.there_prev = (uint8_t)((in_r0.w >> 8) & 0xff); rec.pad = 0;
-            rec.tt = __int_as_float(in_r1.x); rec.cl = __int_as_float(in_r1.y);
-            rec.hn = __int_as_float(in_r1.z); rec.lax = __int_as_float(in_r1.w);
+            const EvRec rec = decode_rec(reinterpret_cast<const int4*>(stp + kPfStR0)[j],
+                                         reinterpret_cast<const int4*>(stp + kPfStR1)[j]);
             o_soc = reinterpret_cast<const double*>(stp + kPfStSoc)[j];
             o_sdeg = reinterpret_cast<const double*>(stp + kPfStSdeg)[j];
             const double soh = reinterpret_cast<const double*>(stp + kPfStSoh)[j];
@@ -1528,7 +1496,8 @@ __global__ void __maxnreg__(kPfMaxReg) fleet_step_pf_kernel(const StepParams p) 
             write_ev_obs<kNorm, kAux>(p, orow, n, o_soc, o_hl, rec, flip);
             // time-only part of the observation: element n of this env's header row (+ the rest when N < H)
             if (n < H) orow[hpos] = hv0;
-            for (int q = n + N; q < H; q += N) orow[hdr_pos(q)] = ld_keep_f32(p.hdr + (size_t)t1 * p.hdr_stride + q, keep);
+            for (int q = n + N; q < H; q += N)
+                orow[hdr_pos<kAux>(p.Ha, N, q)] = ld_keep_f32(p.hdr + (size_t)t1 * p.hdr_stride + q, keep);
         }
         // even N: the two vehicles of a lane pair (same env) are added here, even lane + odd lane
         if (pair) {
@@ -1664,7 +1633,7 @@ __global__ void __launch_bounds__(kT, kT == 32 ? 2 * kPostMinCtas : kPostMinCtas
         int t0 = 0;
         if (wf & WL_RESET) {
             PT_COUNT(13, 1);
-            t0 = p.next_start ? p.next_start[e] : draw_start(p.seed, p.start_lo, p.start_hi, p.env_id_offset + e, ev.z);
+            t0 = episode_start(p, p.next_start, e, ev.z);
             if (mine) reset_slot<kNorm, kAux>(p, e, n, t0, p.obs ? p.obs + (size_t)e * p.D : nullptr, !p.carry);
             PT_MARK(14);
         }
@@ -1677,8 +1646,7 @@ __global__ void __launch_bounds__(kT, kT == 32 ? 2 * kPostMinCtas : kPostMinCtas
             }
             if (last) {
                 if (wf & WL_RESET) {
-                    p.env4[e] = make_int4(t0, t0, ev.z + 1, 0);
-                    p.env_f64[(size_t)EF_EP_RETURN * p.E + e] = 0;
+                    begin_episode(p, e, t0, ev.z);
                 } else if (p.rf_on) {
                     p.env4[e] = make_int4(ev.x, ev.y, ev.z, k_now);    // samples up to k_now are consumed
                 }
@@ -1737,18 +1705,15 @@ __global__ void __launch_bounds__(kThreads) fleet_reset_kernel(const StepParams 
         const int b = j / N, n = j - b * N;
         const int e = e0 + b;
         if (p.mask && !p.mask[e]) continue;
-        const int4 ev = p.env4[e];
-        const int t0 = p.start_idx ? p.start_idx[e] : draw_start(p.seed, p.start_lo, p.start_hi, p.env_id_offset + e, ev.z);
+        const int t0 = episode_start(p, p.start_idx, e, p.env4[e].z);
         reset_slot<kNorm, kAux>(p, e, n, t0, p.obs ? p.obs + (size_t)e * p.D : nullptr, !p.carry);
     }
     __syncthreads();  // all slots have read env4 before it is rewritten
     if (threadIdx.x < nb) {
         const int e = e0 + threadIdx.x;
         if (!(p.mask && !p.mask[e])) {
-            const int4 ev = p.env4[e];
-            const int t0 = p.start_idx ? p.start_idx[e] : draw_start(p.seed, p.start_lo, p.start_hi, p.env_id_offset + e, ev.z);
-            p.env4[e] = make_int4(t0, t0, ev.z + 1, 0);
-            p.env_f64[(size_t)EF_EP_RETURN * p.E + e] = 0;
+            const int ep_count = p.env4[e].z;
+            begin_episode(p, e, episode_start(p, p.start_idx, e, ep_count), ep_count);
         }
     }
 }
@@ -2555,7 +2520,7 @@ int fleet_create(const FleetConsts* consts, const FleetTables* tb, int32_t num_e
                 p.pf_pair = (N & 1) ? 0 : 1;
                 p.pf_cslots = pf_contrib_slots(pfB, N);
                 p.pf_cper = p.pf_pair ? N / 2 : N;
-                p.pf_envs_b = (int)align16((size_t)pfB * sizeof(PfEnv));
+                p.pf_envs_b = (int)align16((size_t)pfB * sizeof(EnvS));
                 p.pf_contrib_b = (int)align16((size_t)kNQ * p.pf_cslots * 8);
                 p.pf_obs_b = (int)align16((size_t)pfB * h->D * 4 + 12);     // + the destination's phase inside a 16-byte line
                 p.pf_off_contrib = kPfEnvs * p.pf_envs_b;
