@@ -34,12 +34,14 @@ def knobs(monkeypatch):
     return set_knobs
 
 
-def make_case(name, n_evs, days=12, use_case="lmd", sph=4, episode_hours=24, two_trips=False, over=None):
-    """(consts, tables) of a synthetic fleet; the tables' seed is derived from `name`, so a case is stable across runs."""
+def make_case(name, n_evs, days=12, use_case="lmd", sph=4, episode_hours=24, two_trips=False, over=None,
+              table_target=0.85):
+    """(consts, tables) of a synthetic fleet; the tables' seed is derived from `name`, so a case is stable across runs.
+    table_target: the target SOC the tables' SOC_on_return is derived from (independent of the constants' target_soc)."""
     over = dict(over or {})
     cap0 = dict(lmd=60.0, ut=50.0, ct=16.7)[use_case]
     tables, T = make_tables(n_evs=n_evs, days=days, sph=sph, seed=zlib.crc32(name.encode()) % 1000, two_trips=two_trips,
-                            cap=cap0)
+                            cap=cap0, target_soc=table_target)
     if not over.get("include_building", 1):
         tables = dict(tables, load=None)
     if not over.get("include_pv", 1):

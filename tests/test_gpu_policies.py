@@ -20,15 +20,33 @@ def _inputs(use_case, n):
     return FleetInputs(sched, price, tariff, load, pv)
 
 
-@pytest.mark.parametrize("use_case,n_evs", [("lmd", 6), ("ct", 4)])
+# id -> (use case, N, env_config overrides).  1h: a 1-hour grid, where the night window opens only at charging minute 0
+# (target 1.0 puts it at 23:00 for this schedule); 33: the (env, EV) index i / N crosses a warp inside an env; tuned: the
+# distributed rule and night_params read target_soc and charging_eff, the fleet's trajectory obc_max_power (below evse).
+CASES = {
+    "lmd-6": ("lmd", 6, {}),
+    "ct-4": ("ct", 4, {}),
+    "ut-5": ("ut", 5, {}),
+    "lmd-4-1h": ("lmd", 4, dict(freq="1h", minutes=60, time_steps_per_hour=1, target_soc=1.0)),
+    "lmd-33": ("lmd", 33, {}),
+    "ct-6-tuned": ("ct", 6, dict(target_soc=0.95, charging_eff=0.82, obc_max_power=3.0)),
+}
+
+
+@pytest.mark.parametrize("case", list(CASES))
 @pytest.mark.parametrize("policy", ["uncontrolled", "distributed", "night"])
-def test_policy_actions_match_reference_rules(use_case, n_evs, policy):
+def test_policy_actions_match_reference_rules(case, policy):
     from fleetrl_b200 import FleetVecEnv
-    cfg = default_config(use_case, time_picker="random", end_cutoff=10, episode_length=48 if use_case == "ct" else 24)
+    use_case, n_evs, over = CASES[case]
+    cfg = default_config(use_case, time_picker="random", end_cutoff=10, episode_length=48 if use_case == "ct" else 24,
+                         **over)
     E = 24
     env = FleetVecEnv(cfg, E, inputs=_inputs(use_case, n_evs), output="torch", seed=9)
     c, tb = env.built.consts, env.built.tables
     env.reset()
+    for k, v in over.items():
+        if hasattr(c, k):
+            assert getattr(c, k) == v, k
     npar = night_params(env.built)
     assert 0 <= npar.charging_hour <= 23 and npar.charging_minute in (0, 15, 30, 45)
     night = [opol.NightPolicy(c, tb, npar.charging_hour, npar.charging_minute, npar.max_hours) for _ in range(E)]
