@@ -58,9 +58,13 @@ enum { Q_REWARD = 0, Q_CASH, Q_ATH, Q_MISS, Q_NVIOL };
 // per-time flags
 constexpr uint32_t TF_TRIGGER = 1u;  // hour == 14 && minute == 45     fleet_environment.py:665
 constexpr uint32_t TF_LUNCH = 2u;    // 11 < hour < 15                 fleet_environment.py:538
+// StepRow::flags_next carries, above its TF_* bits, the distance from row t to the first 14:45 row at or after t + 2
+constexpr int TF_DIST_SHIFT = 8;
+constexpr uint32_t TF_DIST_NONE = 0xffffffu;   // no such row (saturated)
 
 // per-env tile flags
-constexpr int EF_FROZEN = 1, EF_DONE = 2, EF_TRIGGER = 4, EF_LUNCH = 8, EF_RESET = 16;
+//   EF_EVAL_AHEAD   a daily evaluation remains in the episode after this step's (next 14:45 row at or after t + 2 <= t_fin)
+constexpr int EF_FROZEN = 1, EF_DONE = 2, EF_TRIGGER = 4, EF_LUNCH = 8, EF_RESET = 16, EF_EVAL_AHEAD = 32;
 
 // One (time, vehicle) schedule record, 32 bytes = one L2 sector: SOC_on_return, time_left, There at this row and
 // at the previous row, and the auxiliary observation terms of observer_bl_pv.py:85-91 for the un-raised target
@@ -84,7 +88,7 @@ struct __align__(16) StepRow {
     double gml;       // grid_connection - load[t]                                load_calculation.py:93
     double pvv;       // pv[t]
     uint32_t flags;       // TF_* of row t
-    uint32_t flags_next;  // TF_* of row t+1
+    uint32_t flags_next;  // TF_* of row t+1 | distance to the first 14:45 row >= t+2 << TF_DIST_SHIFT
 };
 static_assert(sizeof(StepRow) == 64, "StepRow must be 64 bytes");
 
@@ -111,7 +115,9 @@ struct StepParams {
     const StepRow* step_row;  // [T]
     const float* hdr;         // [T][hdr_stride]
     // state
-    int4* env4;               // [E] {t, t_start, ep_count, k_done}: k_done = newest history sample the rainflow state has consumed
+    int4* env4;               // [E] {t, t_start, ep_count, k_done}: k_done = newest history sample the rainflow state has consumed;
+                              // once no daily evaluation remains in the episode the ring may wrap over unconsumed samples
+                              // and k_done lag by more than R - 1 (wl_flags): nothing reads them before the reset
     double* soc;              // [E][N]
     float* hl;                // [E][N]
     double* soh;              // [E][N]
@@ -876,7 +882,7 @@ __device__ __forceinline__ void ev_slot_step(const StepParams& p, const EnvS& es
 constexpr int WL_TRIGGER = 1, WL_RESET = 2, WL_FLUSH = 4;
 // Entries with a daily evaluation are by far the longest (consumption + residue stress + fade): they are pushed from the
 // front of the list and fetched first by the post kernel, everything else from the back, so that the kernel does not end
-// with one late-started evaluation.  Flush-only entries (most entries) go to a list of their own, which the post kernel
+// with one late-started evaluation.  Flush-only entries (most entries; wl_flags) go to a list of their own, which the post kernel
 // works through in units of 32 vehicles per warp after the other entries; they carry the env's k_done and k_now, so the
 // post kernel never reads env4 of an env whose k_done another warp of the same launch may already have advanced.
 __device__ __forceinline__ void wl_push(const StepParams& p, int e, int wf, int k_done, int k_now) {
@@ -887,11 +893,14 @@ __device__ __forceinline__ void wl_push(const StepParams& p, int e, int wf, int 
 __device__ __forceinline__ int2 wl_fetch(const StepParams& p, int w, int n_front) {
     return p.wl[w < n_front ? w : p.E - 1 - (w - n_front)];
 }
-// Work-list flags of an env whose step k (history sample k+1) has just been taken.  WL_FLUSH: with the next sample the
-// ring would hold more than R rows (samples k_done .. k+2), so the pending ones are consumed now.
+// Work-list flags of an env whose step k (history sample k+1) has just been taken.  The rainflow state is read only by
+// the daily evaluations, and the reset restarts it, so samples are consumed only while an evaluation remains in the
+// episode (EF_EVAL_AHEAD).  Then WL_FLUSH is pushed when with the next sample the ring would hold more than R rows
+// (samples k_done .. k+2), so the pending ones are consumed now.  After the last evaluation the ring wraps over unconsumed samples and k_done falls behind; the rule is monotone within
+// an episode, so no consumer ever starts from such a k_done.
 __device__ __forceinline__ int wl_flags(const StepParams& p, int env_flags, int k, int k_done) {
     int wf = ((env_flags & EF_TRIGGER) ? WL_TRIGGER : 0) | ((env_flags & EF_RESET) ? WL_RESET : 0);
-    if (p.rf_on && k + 1 - k_done >= p.R - 1) wf |= WL_FLUSH;
+    if (p.rf_on && (env_flags & EF_EVAL_AHEAD) && k + 1 - k_done >= p.R - 1) wf |= WL_FLUSH;
     return wf;
 }
 
@@ -912,6 +921,9 @@ __device__ __forceinline__ int stage_env_scratch(const StepParams& p, EnvS& es, 
         if (env4.x + 1 == t_fin) fl |= auto_reset ? EF_DONE | EF_RESET : EF_DONE;
         if ((fn & TF_TRIGGER) && p.calc_deg) fl |= EF_TRIGGER;
         if (fn & TF_LUNCH) fl |= EF_LUNCH;
+        // the next 14:45 row at or after t + 2, from the row actually read (past T - 2 there is none: saturated)
+        const int dist = (int)(fn >> TF_DIST_SHIFT);
+        if (p.calc_deg && dist != (int)TF_DIST_NONE && min(env4.x, p.T - 2) + dist <= t_fin) fl |= EF_EVAL_AHEAD;
     }
     es.flags = fl;
     es.S = __hiloint2double(r0.y, r0.x); es.F_cr = __hiloint2double(r0.w, r0.z);
@@ -2081,6 +2093,9 @@ int64_t fleet_state_bytes(FleetHandle* h) {
     return (int64_t)n;
 }
 
+// The blob holds the state as the kernels left it: an env exported after the last daily evaluation of its episode may
+// hold a history ring that has wrapped over samples the rainflow state never consumed (k_done < k_now - R + 1).  Nothing
+// reads them before the env's next reset, so an import continues it exactly.
 int fleet_export_state(FleetHandle* h, void* dst_host, void* stream) {
     if (!h || !dst_host) return FLEET_E_INVALID;
     CUDA_TRY(h, cudaSetDevice(h->device));
@@ -2294,6 +2309,9 @@ int fleet_create(const FleetConsts* consts, const FleetTables* tb, int32_t num_e
     }
     std::vector<StepRow> rows((size_t)T);
     const double spot_offset = c.fixed_markup / 1000;                                    // ev_charger.py:35
+    // next_trig[t]: the first 14:45 row at or after t (T: none)
+    std::vector<int> next_trig((size_t)T + 2, T);
+    for (int t = T - 1; t >= 0; t--) next_trig[t] = (tb->hour[t] == 14 && tb->minute[t] == 45) ? t : next_trig[t + 1];
     for (int t = 0; t < T; t++) {
         StepRow& r = rows[t];
         double connected = 0;
@@ -2314,7 +2332,9 @@ int fleet_create(const FleetConsts* consts, const FleetTables* tb, int32_t num_e
             return f;
         };
         r.flags = tf(t);
-        r.flags_next = tf(t + 1 < T ? t + 1 : T - 1);
+        const int nt = next_trig[t + 2 < T ? t + 2 : T];
+        const uint32_t dist = nt < T ? std::min((uint32_t)(nt - t), TF_DIST_NONE) : TF_DIST_NONE;
+        r.flags_next = tf(t + 1 < T ? t + 1 : T - 1) | dist << TF_DIST_SHIFT;
     }
     const int hdr_stride = ((Ha + Hb + 3) / 4) * 4 > 0 ? ((Ha + Hb + 3) / 4) * 4 : 4;
     std::vector<float> hdr((size_t)T * hdr_stride, 0.f);
@@ -2373,7 +2393,8 @@ int fleet_create(const FleetConsts* consts, const FleetTables* tb, int32_t num_e
     CUDA_TRY(h, cudaMemcpy(d_hdr, hdr.data(), hdr.size() * sizeof(float), cudaMemcpyHostToDevice));
 
     // History ring and incremental rainflow geometry.  Samples are only needed until the post kernel has consumed them
-    // (at the daily trigger, or when the ring is about to wrap), so R rows suffice for any episode length.
+    // (at the daily trigger, or when the ring is about to wrap while an evaluation remains in the episode), so R rows
+    // suffice for any episode length.
     bool any_trigger = false;
     for (int t = 0; t < T; t++) any_trigger = any_trigger || (rows[t].flags & TF_TRIGGER);
     const bool rf_on = c.calc_degradation && c.deg_mode == FLEET_DEG_SEI && any_trigger;   // (no 14:45 row, e.g. 1-h grids: never evaluated)
