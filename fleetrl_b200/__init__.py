@@ -16,6 +16,9 @@ def __getattr__(name):  # lazy: importing the package must not require torch / C
     if name in ("FleetRolloutBuffer", "RolloutBufferSamples", "collect_rollouts"):
         from . import rollout
         return getattr(rollout, name)
+    if name in ("FleetMlpPolicy", "ppo_loss", "ppo_train"):
+        from . import ppo
+        return getattr(ppo, name)
     if name in ("build_fleet", "FleetInputs"):
         from . import tables
         return getattr(tables, name)

@@ -27,6 +27,7 @@ EXPORTS = [
     "fleet_norm_create", "fleet_norm_destroy", "fleet_norm_set_flags", "fleet_norm_moments_len", "fleet_norm_moments",
     "fleet_norm_apply", "fleet_norm_reset_returns", "fleet_norm_get_state", "fleet_norm_set_state", "fleet_norm_last_error",
     "fleet_rollout_add", "fleet_rollout_gae", "fleet_rollout_gather", "fleet_rollout_last_error",
+    "fleet_ppo_workspace_bytes", "fleet_ppo_log_prob", "fleet_ppo_loss", "fleet_ppo_loss_backward", "fleet_ppo_last_error",
 ]
 
 
@@ -39,6 +40,19 @@ class FleetRolloutBuf(C.Structure):
     _fields_ = [(n, C.c_int32) for n in ("buffer_size", "num_envs", "obs_dim", "action_dim")] + \
                [(n, C.c_void_p) for n in ("observations", "actions", "rewards", "episode_starts", "values", "log_probs",
                                           "advantages", "returns")]
+
+
+class FleetPpoBatch(C.Structure):
+    """struct FleetPpoBatch of fleetstep.h: one minibatch's sizes and device pointers."""
+    _fields_ = [("batch_size", C.c_int64), ("action_dim", C.c_int32), ("reserved", C.c_int32)] + \
+               [(n, C.c_void_p) for n in ("mean", "log_std", "actions", "values", "old_log_prob", "old_values",
+                                          "advantages", "returns")]
+
+
+class FleetPpoParams(C.Structure):
+    """struct FleetPpoParams of fleetstep.h (clip_range_vf < 0 means None)."""
+    _fields_ = [(n, C.c_double) for n in ("clip_range", "clip_range_vf", "ent_coef", "vf_coef")] + \
+               [("normalize_advantage", C.c_int32), ("reserved", C.c_int32)]
 
 
 def load_library(path: str = LIB_PATH):
@@ -107,6 +121,14 @@ def load_library(path: str = LIB_PATH):
     L.fleet_rollout_gather.argtypes = [rb, vp, i64] + [vp] * 7
     L.fleet_rollout_last_error.argtypes = []
     L.fleet_rollout_last_error.restype = C.c_char_p
+    pb, pp = C.POINTER(FleetPpoBatch), C.POINTER(FleetPpoParams)
+    L.fleet_ppo_workspace_bytes.argtypes = [i64, i32]
+    L.fleet_ppo_workspace_bytes.restype = i64
+    L.fleet_ppo_log_prob.argtypes = [pb, vp, vp]
+    L.fleet_ppo_loss.argtypes = [pb, pp, vp, vp, vp, vp, i64, vp]
+    L.fleet_ppo_loss_backward.argtypes = [pb, pp] + [vp] * 6 + [i64, vp]
+    L.fleet_ppo_last_error.argtypes = []
+    L.fleet_ppo_last_error.restype = C.c_char_p
     if L.fleet_abi_version() != ABI_VERSION:
         raise FleetStepError("libfleetstep.so ABI version does not match fleetrl_b200/_abi.py")
     _LIB = L

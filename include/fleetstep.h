@@ -414,6 +414,73 @@ int fleet_rollout_gather(const FleetRolloutBuf* b, const int64_t* flat_idx_dev, 
 /* Message of the calling thread's last failing fleet_rollout_* call. */
 const char* fleet_rollout_last_error(void);
 
+/*
+ * FleetPpo — the per-minibatch loss of SB3 2.3.2's PPO.train (stable_baselines3/ppo/ppo.py) for a diagonal Gaussian
+ * policy (common/distributions.py, DiagGaussianDistribution), forward and backward.  Stateless: the caller owns every
+ * array, including a workspace of fleet_ppo_workspace_bytes(B, N) bytes, 256-byte aligned and zero-filled before its
+ * first use (each call leaves it reusable).  No call synchronises the host, no kernel uses floating-point atomics, and
+ * every output is bit-identical from call to call: reductions run in float64 over fixed chunks of rows, combined in a
+ * fixed order by the last CTA of each launch.  Offsets are 64-bit.  FLEET_E_INVALID for bad sizes, NULL pointers,
+ * clip_range <= 0 or a workspace that is too small; fleet_ppo_last_error() returns the calling thread's message.
+ * All arrays are float32 on the device.
+ */
+typedef struct FleetPpoBatch {
+    int64_t batch_size;          /* B                                                                          */
+    int32_t action_dim;          /* N                                                                          */
+    int32_t reserved;
+    const float* mean;           /* [B][N]  mean_actions of the policy                                          */
+    const float* log_std;        /* [N]     the policy's state-independent log_std                              */
+    const float* actions;        /* [B][N]  RolloutBufferSamples.actions                                        */
+    const float* values;         /* [B]     the value head's output                                            */
+    const float* old_log_prob;   /* [B]     .old_log_prob                                                       */
+    const float* old_values;     /* [B]     .old_values (read only when clip_range_vf >= 0)                     */
+    const float* advantages;     /* [B]     .advantages                                                         */
+    const float* returns;        /* [B]     .returns                                                            */
+} FleetPpoBatch;
+
+typedef struct FleetPpoParams {
+    double clip_range;           /* > 0                                                                         */
+    double clip_range_vf;        /* < 0: None                                                                   */
+    double ent_coef, vf_coef;
+    int32_t normalize_advantage; /* applied only when B > 1, as SB3 does                                        */
+    int32_t reserved;
+} FleetPpoParams;
+
+/* Bytes of workspace fleet_ppo_loss and fleet_ppo_loss_backward need for B rows of N actions (0 for sizes < 1). */
+int64_t fleet_ppo_workspace_bytes(int64_t batch_size, int32_t action_dim);
+
+/* DiagGaussianDistribution.log_prob (distributions.py) over Normal(mean, ones_like(mean) * exp(log_std)) (torch's
+ * Normal.log_prob): lp[i] = sum_n ( -(a - mu)^2 / (2 sigma^2) - log(sigma) - log(sqrt(2 pi)) ) with sigma = exp(log_std),
+ * each term in float32 in torch's order, the sum over n in float64 in a fixed order, rounded once.  Reads mean, log_std
+ * and actions of the batch; writes log_prob_out [B].  fleet_ppo_loss computes the same bits for the same inputs. */
+int fleet_ppo_log_prob(const FleetPpoBatch* b, float* log_prob_out, void* stream);
+
+/* The loss of one minibatch of PPO.train (ppo.py), in two launches:
+ *   A = advantages, normalised when normalize_advantage and B > 1: (A - m) / (s + 1e-8) with the mean m and the
+ *       unbiased std s reduced in float64 and rounded to float32;
+ *   ratio = exp(log_prob - old_log_prob);  policy_loss = -mean(min(A * ratio, A * clamp(ratio, 1 - eps, 1 + eps)));
+ *   values_pred = values, or old_values + clamp(values - old_values, -c, c) when clip_range_vf = c >= 0;
+ *   value_loss = mean((returns - values_pred)^2);  entropy_loss = -mean(entropy) = -sum_n (0.5 + 0.5 log 2pi + log sigma_n);
+ *   loss = policy_loss + ent_coef * entropy_loss + vf_coef * value_loss  -> *loss_out (float32, device).
+ * Adds this minibatch's policy_loss, value_loss, entropy_loss, clip_fraction (mean of |ratio - 1| > eps) and approx_kl
+ * (mean((ratio - 1) - log_ratio)) to stats_acc[0..4] (float64, device).  Writes sample_coef [2][B]: d loss / d log_prob
+ * and d loss / d values of every row, which fleet_ppo_loss_backward reads. */
+int fleet_ppo_loss(const FleetPpoBatch* b, const FleetPpoParams* p, float* loss_out, double* stats_acc,
+                   float* sample_coef, void* workspace, int64_t workspace_bytes, void* stream);
+
+/* The gradient of fleet_ppo_loss as torch autograd gives it on SB3's composition (clamp passes the gradient on its
+ * closed interval, minimum splits a tie in half, the normalised advantage carries none), in one launch.  grad_loss is
+ * read from device memory; with g_i = grad_loss * d loss / d log_prob_i:
+ *   grad_mean [B][N] = g_i (a - mu) / sigma^2;   grad_values [B] = grad_loss * d loss / d values_i;
+ *   grad_log_std [N] = sum_i g_i ((a - mu)^2 / sigma^2 - 1) - grad_loss * ent_coef  (float64 column sums).
+ * b and p must be those of the fleet_ppo_loss call that wrote sample_coef. */
+int fleet_ppo_loss_backward(const FleetPpoBatch* b, const FleetPpoParams* p, const float* grad_loss,
+                            const float* sample_coef, float* grad_mean, float* grad_log_std, float* grad_values,
+                            void* workspace, int64_t workspace_bytes, void* stream);
+
+/* Message of the calling thread's last failing fleet_ppo_* call. */
+const char* fleet_ppo_last_error(void);
+
 #ifdef __cplusplus
 }
 #endif
