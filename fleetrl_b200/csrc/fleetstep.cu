@@ -1,7 +1,8 @@
 // fleetstep.cu — B200 (sm_100a) implementation of the FleetRL environment step behind include/fleetstep.h.
 //
 // Two launches per fleet_step call, on the caller's stream:
-//   step kernel   fleet_step_pf_kernel (persistent, warp-specialised, software-pipelined; auto-reset on, 8 <= N <= 256) or
+//   step kernel   fleet_step_pf_kernel (persistent, warp-specialised, software-pipelined; auto-reset on, 8 <= N <= 256;
+//                 a generic instance and one compiled for the cfg2 fleet shape) or
 //                 fleet_step_kernel (generic: any N, frozen envs): EvCharger.charge + LoadCalculation.check_violation +
 //                 ScoreConfig penalties + time advance + departure/arrival logic + Observer/Normalization observation
 //                 assembly for E envs x N EVs; appends the new soc_deg sample to a small per-env ring and pushes envs that
@@ -990,7 +991,7 @@ __device__ __forceinline__ void finalise_env(const StepParams& p, const EnvS& es
 
 // Shared-memory layout (dynamic): EnvS envs[B] | double contrib[kNQ][slots] | double sums[kNQ][B] |
 //                                 float obs_tile[B][D] (16-byte aligned)
-__host__ __device__ inline size_t align16(size_t x) { return (x + 15) & ~(size_t)15; }
+__host__ __device__ constexpr size_t align16(size_t x) { return (x + 15) & ~(size_t)15; }
 __host__ __device__ inline size_t smem_envs_bytes(int B) { return align16((size_t)B * sizeof(EnvS)); }
 __host__ __device__ inline size_t smem_obs_offset(int B, int N) {
     return align16(smem_envs_bytes(B) + (size_t)kNQ * B * N * 8 + (size_t)kNQ * B * 8);
@@ -1170,11 +1171,66 @@ constexpr int kPfStA32 = 0, kPfStHl = 4 * kPfSlots, kPfStHv = 8 * kPfSlots, kPfS
 constexpr int kPfStages = 2;  // input stages: the copies of a tile are issued two tiles ahead
 constexpr int kPfOut = 3;     // output buffers (contributions + obs tile): the epilogue may lag two tiles behind
 constexpr int kPfEnvs = 4;    // env-scratch buffers: staged three tiles ahead
-// Even N: neighbouring vehicles' contributions are added in the compute warp (one shuffle), halving the buffer.
-__host__ __device__ inline int pf_contrib_slots(int B, int N) { return (N & 1) ? B * N : (B * N) / 2; }
-__host__ __device__ inline size_t pf_smem_bytes(int B, int N, int D) {
-    return align16(kPfEnvs * align16((size_t)B * sizeof(EnvS)) + kPfOut * align16((size_t)kNQ * pf_contrib_slots(B, N) * 8) +
-                   2 * align16((size_t)kNQ * B * 8) + kPfOut * align16((size_t)B * D * 4 + 12)) + (size_t)kPfStages * kPfStageBytes;
+// Tile geometry and shared-memory layout of the pf kernel for N vehicles, observation width D and a history ring of R
+// rows: filled into StepParams by fleet_create, and folded to literals inside a shape-specialised instance.
+struct PfLayout {
+    int B;                    // envs per tile
+    int pair;                 // even N: neighbouring vehicles' contributions are added in the compute warp (one shuffle),
+    int cslots, cper;         // halving the buffer; contribution entries per quantity and tile / per env
+    unsigned int tile_hist;   // B * R * N: history elements per tile
+    int envs_b, contrib_b, obs_b;                  // bytes of one env-scratch / contribution / obs buffer
+    int off_contrib, off_sums, off_obs, off_stage;
+    size_t smem;              // dynamic shared memory
+};
+__host__ __device__ constexpr PfLayout pf_layout(int N, int D, int R) {
+    PfLayout l{};
+    l.B = kPfSlots / N;
+    l.pair = (N & 1) ? 0 : 1;
+    l.cslots = l.pair ? (l.B * N) / 2 : l.B * N;
+    l.cper = l.pair ? N / 2 : N;
+    l.tile_hist = (unsigned int)((size_t)l.B * R * N);
+    l.envs_b = (int)align16((size_t)l.B * sizeof(EnvS));
+    l.contrib_b = (int)align16((size_t)kNQ * l.cslots * 8);
+    l.obs_b = (int)align16((size_t)l.B * D * 4 + 12);   // + the destination's phase inside a 16-byte line
+    l.off_contrib = kPfEnvs * l.envs_b;
+    l.off_sums = l.off_contrib + kPfOut * l.contrib_b;
+    l.off_obs = l.off_sums + 2 * (int)align16((size_t)kNQ * l.B * 8);
+    l.off_stage = (int)align16((size_t)l.off_obs + (size_t)kPfOut * l.obs_b);
+    l.smem = (size_t)l.off_stage + (size_t)kPfStages * kPfStageBytes;
+    return l;
+}
+
+// Compile-time shape of a pf kernel instance.  All zero: any fleet, sizes read from StepParams.  Otherwise the instance
+// runs only fleets of exactly N vehicles, observation width D, header Ha + Hb and a history ring of R rows, and every
+// size, index and shared-memory offset derived from them is a literal (a fifth fewer instructions).
+template <int kN, int kD, int kHa, int kHb, int kR>
+struct PfShape {
+    static constexpr int N = kN, D = kD, Ha = kHa, Hb = kHb, R = kR;
+};
+using PfAnyShape = PfShape<0, 0, 0, 0, 0>;
+// bench.py's metric workload (cfg2): last-mile-delivery fleet of 50 EVs, full observer (price look-ahead 8, building /
+// PV look-ahead 4, auxiliary terms, not normalised), rainflow-SEI with the default 16-row history ring
+using PfCfg2Shape = PfShape<50, 388, 28, 10, 16>;
+
+// The kernel's parameter block with the geometry of a specialised shape overwritten by literals (a local copy: every
+// field the kernel reads is still a constant-bank operand, the overwritten ones fold into the code).
+template <class Shape>
+__device__ __forceinline__ StepParams pf_params(const StepParams& pk) {
+    static_assert(Shape::N == 0 || (Shape::N >= 8 && Shape::N <= kPfSlots && Shape::D == 7 * Shape::N + Shape::Ha + Shape::Hb &&
+                                    Shape::R >= 4 && (Shape::R & (Shape::R - 1)) == 0),
+                  "a specialised shape has auxiliary terms (D = 7 N + Ha + Hb) and a power-of-two ring");
+    StepParams p = pk;
+    if constexpr (Shape::N != 0) {
+        constexpr int N = Shape::N, H = Shape::Ha + Shape::Hb;
+        constexpr PfLayout l = pf_layout(N, Shape::D, Shape::R);
+        p.N = N; p.D = Shape::D; p.Ha = Shape::Ha; p.Hb = Shape::Hb; p.hdr_stride = (H + 3) / 4 * 4;
+        p.R = Shape::R; p.Rm = Shape::R - 1; p.RN = (unsigned long long)Shape::R * N;
+        p.n_magic = (unsigned int)((0x100000000ull + N - 1) / N);
+        p.pf_B = l.B; p.pf_pair = l.pair; p.pf_cslots = l.cslots; p.pf_cper = l.cper; p.pf_tile_hist = l.tile_hist;
+        p.pf_envs_b = l.envs_b; p.pf_contrib_b = l.contrib_b; p.pf_obs_b = l.obs_b;
+        p.pf_off_contrib = l.off_contrib; p.pf_off_sums = l.off_sums; p.pf_off_obs = l.off_obs; p.pf_off_stage = l.off_stage;
+    }
+    return p;
 }
 
 __device__ __forceinline__ uint32_t smem_u32(const void* ptr) { return (uint32_t)__cvta_generic_to_shared(ptr); }
@@ -1222,9 +1278,11 @@ __device__ unsigned long long g_pf_trace[10 * 8 * 8];
 #define PF_FLUSH(base) do {} while (0)
 #endif
 // kLog: keep EvCharger's charge_log (fleet_enable_charge_log); a template flag so that the default instance carries
-// neither the extra live register nor the store.
-template <bool kNorm, bool kAux, bool kLog>
-__global__ void __maxnreg__(kPfMaxReg) fleet_step_pf_kernel(const StepParams p) {
+// neither the extra live register nor the store.  Shape: PfAnyShape or a specialised PfShape (fleet_create checks that
+// the fleet matches it).
+template <bool kNorm, bool kAux, bool kLog, class Shape>
+__global__ void __maxnreg__(kPfMaxReg) fleet_step_pf_kernel(const StepParams pk) {
+    const StepParams p = pf_params<Shape>(pk);
     extern __shared__ __align__(16) unsigned char smem_raw[];
     const int N = p.N, B = p.pf_B, D = p.D;
     const int cstride = B * N;
@@ -1913,6 +1971,7 @@ struct FleetHandle {
     std::string err;
     size_t smem_step = 0, smem_post = 0, smem_pf = 0;
     int grid_pf = 0, use_pf = 0;
+    int pf_cfg2 = 0;                    // the fleet has the shape of the specialised pf instance (PfCfg2Shape)
     int grid = 0, grid_post = 0, need_post = 0, num_sms = 0, post_threads = kPostThreads;
     int max_smem_optin = 0;
     double* charge_log_buf = nullptr;   // fleet_enable_charge_log
@@ -1992,13 +2051,21 @@ StepKernel pick_step(const FleetHandle* h) {
     if (h->c.normalize) return h->c.aux ? fleet_step_kernel<true, true> : fleet_step_kernel<true, false>;
     return h->c.aux ? fleet_step_kernel<false, true> : fleet_step_kernel<false, false>;
 }
+// The fleet has exactly the compile-time shape S and the flags of its instance (kNorm = false, kAux = true).
+template <class S>
+bool pf_shape_is(const FleetHandle* h) {
+    const StepParams& p = h->p;
+    return !h->c.normalize && h->c.aux && p.N == S::N && p.D == S::D && p.Ha == S::Ha && p.Hb == S::Hb && p.R == S::R;
+}
 StepKernel pick_pf(const FleetHandle* h, bool log) {
+    using A = PfAnyShape;
+    if (h->pf_cfg2 && !log) return fleet_step_pf_kernel<false, true, false, PfCfg2Shape>;
     if (log) {
-        if (h->c.normalize) return h->c.aux ? fleet_step_pf_kernel<true, true, true> : fleet_step_pf_kernel<true, false, true>;
-        return h->c.aux ? fleet_step_pf_kernel<false, true, true> : fleet_step_pf_kernel<false, false, true>;
+        if (h->c.normalize) return h->c.aux ? fleet_step_pf_kernel<true, true, true, A> : fleet_step_pf_kernel<true, false, true, A>;
+        return h->c.aux ? fleet_step_pf_kernel<false, true, true, A> : fleet_step_pf_kernel<false, false, true, A>;
     }
-    if (h->c.normalize) return h->c.aux ? fleet_step_pf_kernel<true, true, false> : fleet_step_pf_kernel<true, false, false>;
-    return h->c.aux ? fleet_step_pf_kernel<false, true, false> : fleet_step_pf_kernel<false, false, false>;
+    if (h->c.normalize) return h->c.aux ? fleet_step_pf_kernel<true, true, false, A> : fleet_step_pf_kernel<true, false, false, A>;
+    return h->c.aux ? fleet_step_pf_kernel<false, true, false, A> : fleet_step_pf_kernel<false, false, false, A>;
 }
 template <int kT>
 StepKernel pick_post_t(const FleetHandle* h) {
@@ -2526,7 +2593,9 @@ int fleet_create(const FleetConsts* consts, const FleetTables* tb, int32_t num_e
         const bool want = !force || strcmp(force, "pf") == 0;
         const int pfB = kPfSlots / N;
         if (want && c.auto_reset && N >= 8 && pfB >= 1 && pfB <= 32) {   // the epilogue warps use one lane per env of a tile
-            const size_t smpf = pf_smem_bytes(pfB, N, h->D);
+            const PfLayout l = pf_layout(N, h->D, R);
+            const size_t smpf = l.smem;
+            h->pf_cfg2 = pf_shape_is<PfCfg2Shape>(h) ? 1 : 0;
             int per_sm = 0;
             if ((int64_t)smpf <= (int64_t)h->max_smem_optin &&
                 cudaFuncSetAttribute(pick_pf(h, false), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smpf) == cudaSuccess &&
@@ -2534,20 +2603,20 @@ int fleet_create(const FleetConsts* consts, const FleetTables* tb, int32_t num_e
                 cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, pick_pf(h, true), kPfThreads, smpf) == cudaSuccess && per_sm >= 1) {
                 h->smem_pf = smpf;
                 const int ntiles = (E + pfB - 1) / pfB;
-                p.pf_B = pfB;
+                p.pf_B = l.B;
                 p.pf_bulk = 1;                                  // (cleared per call when obs / terminal_obs are not 16-byte aligned)
                 p.pf_ntiles = ntiles;
-                p.pf_tile_hist = (unsigned int)((size_t)pfB * p.RN);
-                p.pf_pair = (N & 1) ? 0 : 1;
-                p.pf_cslots = pf_contrib_slots(pfB, N);
-                p.pf_cper = p.pf_pair ? N / 2 : N;
-                p.pf_envs_b = (int)align16((size_t)pfB * sizeof(EnvS));
-                p.pf_contrib_b = (int)align16((size_t)kNQ * p.pf_cslots * 8);
-                p.pf_obs_b = (int)align16((size_t)pfB * h->D * 4 + 12);     // + the destination's phase inside a 16-byte line
-                p.pf_off_contrib = kPfEnvs * p.pf_envs_b;
-                p.pf_off_sums = p.pf_off_contrib + kPfOut * p.pf_contrib_b;
-                p.pf_off_obs = p.pf_off_sums + 2 * (int)align16((size_t)kNQ * pfB * 8);
-                p.pf_off_stage = (int)align16((size_t)p.pf_off_obs + (size_t)kPfOut * p.pf_obs_b);
+                p.pf_tile_hist = l.tile_hist;
+                p.pf_pair = l.pair;
+                p.pf_cslots = l.cslots;
+                p.pf_cper = l.cper;
+                p.pf_envs_b = l.envs_b;
+                p.pf_contrib_b = l.contrib_b;
+                p.pf_obs_b = l.obs_b;
+                p.pf_off_contrib = l.off_contrib;
+                p.pf_off_sums = l.off_sums;
+                p.pf_off_obs = l.off_obs;
+                p.pf_off_stage = l.off_stage;
                 const int g = prop.multiProcessorCount * per_sm;
                 h->grid_pf = g < ntiles ? g : ntiles;
                 // FLEETSTEP_PF_GRID=G (diagnostic, G >= 1) caps the persistent grid so that every CTA runs many tiles: the
